@@ -64,6 +64,9 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=0, help="filters in the CPU sample (0 = auto)")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg4 / strong-split / sustained extras")
     ap.add_argument("--sustained-steps", type=int, default=60)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state the last timed device-resident step left (x_k_k, inlier flags, step "
+                         "statistics, a sample of P_k_k) of rank 0 to DIR/<name>.npy; see dump_outputs()")
     return ap.parse_args()
 
 
@@ -366,6 +369,38 @@ def extra_cfg4(pkg, synth, torch, dev, device_index, peaks):
     return out
 
 
+DUMP_BYTES = 60_000_000   # stays under 64 MB in all, with room for the index arrays
+
+
+def dump_outputs(bank, out_dir):
+    """Writes what a caller of the step receives after the last timed step, so that two builds can be compared output
+    for output on the same seeded workload:
+      x.npy [F, n_max] f64 (x_k_k), flags.npy [F, N] f32 (inlier flag bits), stats.npy [F, 8] f64 (the per-filter step
+      statistics, columns in the order of include/ekfslam.h) for the filters in filters.npy;
+      P.npy [G, R, n_max] f64 (rows P_rows.npy of P_k_k) for the filters in P_filters.npy.
+    Every filter and every row is kept when it fits half of DUMP_BYTES each; otherwise a fixed, seeded sample."""
+    from ekf_slam_b200._lib import STATS_FIELDS
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    B, N, n = bank.B, bank.N, bank.n_max
+    half = DUMP_BYTES // 2
+
+    def sample(total, keep):
+        return np.arange(total) if keep >= total else np.sort(rng.choice(total, keep, replace=False))
+
+    filters = sample(B, half // (8 * n + 4 * N + 8 * len(STATS_FIELDS)))
+    x, _, _ = bank.download_state(want_P=False)
+    st = bank.download_stats()
+    out = {"filters": filters, "x": x[filters], "flags": bank.download_flags()[filters].astype(np.float32),
+           "stats": np.stack([st[k] for k in STATS_FIELDS], axis=1)[filters]}
+    p_filters = sample(B, max(1, half // (8 * n * n)))
+    rows = sample(n, half // (8 * n * len(p_filters)))
+    out.update(P_filters=p_filters, P_rows=rows,
+               P=np.stack([bank.download_state(b0=int(b), nb=1)[1][0][rows] for b in p_filters]))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------
 _REAL_STDOUT = None
 
@@ -474,6 +509,8 @@ def main():
     bank.enable_timing(False)
     stats = bank.download_stats()
     bank.unbind_frame()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(bank, args.dump_outputs)
 
     # ---- timed region: end to end through the host-buffer call ------------------------------
     e2e = None

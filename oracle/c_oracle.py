@@ -33,7 +33,11 @@ def load(build=True):
     if _lib is None:
         so = os.path.join(_HERE, so_name())
         if not os.path.exists(so) and build:
-            subprocess.run(["make", "-C", _HERE, "SO=" + so_name()], check=True, capture_output=True)
+            # built in-tree by __graft_entry__.build(); a host with other CPU flags builds its own copy in a temporary
+            # directory, because the tree may be read-only at run time
+            import tempfile
+            so = os.path.join(tempfile.mkdtemp(prefix="ekf_oracle_"), so_name())
+            subprocess.run(["make", "-C", _HERE, "SO=" + so], check=True, capture_output=True)
         _lib = C.CDLL(so)
         _lib.ekf_oracle_step_batch.restype = C.c_int
         _lib.ekf_oracle_max_threads.restype = C.c_int

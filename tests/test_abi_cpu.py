@@ -3,10 +3,9 @@ declares, and fails loudly (no CPU fallback) when there is no device."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
-import pytest
-
-import ekf_slam_b200 as pkg
 from ekf_slam_b200 import _lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -43,12 +42,17 @@ def test_defaults_match_reference_constants():
 
 
 def test_no_cpu_fallback():
-    lib = _lib.load()
-    if lib.ekfslam_device_count() > 0:
-        pytest.skip("a GPU is visible")
-    with pytest.raises(pkg.EkfSlamError) as e:
-        pkg.FilterBank(2, 4)
-    assert e.value.code == -5 and "no CPU fallback" in str(e.value)
+    """Runs in a child process with every device hidden, so that it also checks this where a GPU is present."""
+    code = ("import ekf_slam_b200 as pkg\n"
+            "try:\n"
+            "    pkg.FilterBank(2, 4)\n"
+            "except pkg.EkfSlamError as e:\n"
+            "    print(e.code, e)\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stderr
+    code, _, msg = r.stdout.strip().partition(" ")
+    assert code == "-5" and "no CPU fallback" in msg, r.stdout
 
 
 def test_argument_validation_without_device():
