@@ -192,13 +192,8 @@ int ekfslam_create(ekfslam_ctx** out, int device, int B, int N_max, int n_max) {
     v.B = B; v.N = N_max; v.nmax = n_max;
     // Row pitch of x / P / G in doubles: a multiple of 32 (256 B).  With the minimal pitch (multiple of 8: 616 at n = 613) the
     // 512-byte row segments of the 64x64 covariance tiles straddle 128-byte lines on every other row; measured on the
-    // HBM-bound hi downdate at the bench shape: pitch 616 -> 4.22 ms, 624 -> 4.08 ms, 640 -> 3.78 ms (EKFSLAM_LD_ALIGN=8|16|32...).
-    {
-        const char* e = getenv("EKFSLAM_LD_ALIGN");
-        int al = e ? atoi(e) : 32;
-        if (al < 8 || (al & 7)) al = 32;
-        v.ld = (n_max + al - 1) / al * al;
-    }
+    // HBM-bound hi downdate at the bench shape: pitch 616 -> 4.22 ms, 624 -> 4.08 ms, 640 -> 3.78 ms.
+    v.ld = (n_max + 31) / 32 * 32;
     v.kmax = 2 * N_max;
     v.n_u = 0;
     c->u_cap = 0;
@@ -763,9 +758,8 @@ int ekfslam_step_graph(ekfslam_ctx* c, int reset, int match_mode) {
     NEED_CTX(c);
     DevView& v = c->v;
     // not capturable: per-kernel timing (event queries), the lock-step Cholesky (host read-back of the largest stacked
-    // size), the host-buffer step's cross-stream events, the lower-triangle mode's host-side state
-    const bool lockstep_shape = v.B < 128 && v.kmax >= 256;
-    if (c->timer || lockstep_shape || c->wait_inputs || c->arm_out) return ekfslam_step(c, reset, match_mode);
+    // size), the host-buffer step's cross-stream events
+    if (c->timer || chol_lockstep(v) || c->wait_inputs || c->arm_out) return ekfslam_step(c, reset, match_mode);
     if (match_mode < 0 || match_mode > 2) return fail(EKFSLAM_ERR_INVALID, "match_mode must be 0, 1 or 2");
     if (v.n_u <= 0) return fail(EKFSLAM_ERR_STATE, "step: no uniform stream uploaded");
     StepGraph* g = (StepGraph*)c->step_graph;

@@ -122,6 +122,11 @@ __host__ __device__ __forceinline__ size_t w_at(int wrows, int t, int c) {
 
 #define EKF_TRI(nic, s) (((nic) * ((nic) + 1)) / 2 + (s))
 
+// The update's Cholesky runs lock-step over all filters (one launch per phase, k_chol_big.cu) for few filters with a
+// large stacked innovation; otherwise one block per filter.  The lock-step path reads the batch's largest stacked size
+// back to the host, so a step that takes it cannot be captured in a CUDA graph (ekfslam_step_graph).
+inline bool chol_lockstep(const DevView& v) { return v.B < 128 && v.kmax >= 256; }
+
 // one process-wide lock for the per-device function-attribute high-water marks (ENSURE_DYN_SMEM)
 inline std::mutex& ekf_attr_mutex() { static std::mutex m; return m; }
 

@@ -11,10 +11,9 @@
 //                   panel-major W layout) on a 4-stage mbarrier ring that keeps running across tile boundaries; 8
 //                   consumer warps issue the DMMAs; 4 epilogue warps prefetch the next P tile into shared memory and
 //                   store the finished tile and its mirror image while the consumers are already in the next K loop.
-//   k_downdate_tile (EKFSLAM_DOWNDATE=tile, and the fallback for shapes whose tile list does not fit the
-//                   persistent kernel's shared memory) one CTA per tile, cp.async (LDGSTS) ring.
+//   k_downdate_tile (the fallback for shapes whose tile list does not fit the persistent kernel's shared memory:
+//                   n_max > 4352 for the li update, n_max > 4608 for the hi update) one CTA per tile, cp.async (LDGSTS) ring.
 #include <cstdlib>
-#include <cstring>
 #include "model.cuh"
 #include "tc_common.cuh"
 
@@ -393,7 +392,7 @@ __device__ __forceinline__ void epi_prefetch_p(double* X, const double* __restri
 // S = stages of the W ring, NX = P tile buffers.  <4,1>: deep ring for long K loops (li update); <2,2>: short K loops
 // (small k, the kernel streams P): the next-but-one P tile is prefetched while the current one is being stored.
 template <int S, int NX>
-__global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int T, int b0, long long total, int M, int mirror) {
+__global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int T, int b0, long long total, int M) {
     extern __shared__ __align__(16) double dsm[];
     double* As = dsm;                                   // [S][TK][TPAD]
     double* Bs = dsm + S * TK * TPAD;           // [S][TK][TPAD]
@@ -589,7 +588,7 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
                     if (j0 + c + 1 < n) *reinterpret_cast<double2*>(o) = val;
                     else if (j0 + c < n) o[0] = val.x;
                 }
-                if (mirror && j0 + r < n) {   // mirror image: row j0 + r of P, columns i0 .. (skipped when only the lower triangle is kept)
+                if (j0 + r < n) {   // mirror image: row j0 + r of P, columns i0 ..
                     double* mrow = P + (size_t)(j0 + r) * ld + i0;
                     if (i0 + lane < n) mrow[lane] = X[lane * XP + r];
                     if (i0 + lane + 32 < n) mrow[lane + 32] = X[(lane + 32) * XP + r];
@@ -620,54 +619,42 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
 
 void launch_downdate(ekfslam_ctx* c, int slot) {
     DevView& v = c->v;
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("EKFSLAM_DOWNDATE");
-        mode = (e && !strcmp(e, "tile")) ? 0 : 2;  // default: persistent warp-specialised kernel
-    }
     const int sms = c->sm_count;   // of the context's own device (a process may drive several GPUs)
     const int nt = (v.nmax + TM - 1) / TM;
     const int T = nt * (nt + 1) / 2;
     KScope ks(c, slot);
-    if (mode == 2) {
-        // ring depth / P buffers by update kind: the hi update usually stacks few rows (short K loops, the kernel
-        // streams P), the li update many.  EKFSLAM_DD_CFG=A|B forces one configuration for both.
-        static int cfgsel = -1;
-        if (cfgsel < 0) {
-            const char* e = getenv("EKFSLAM_DD_CFG");
-            cfgsel = (e && e[0] == 'A') ? 1 : (e && e[0] == 'B') ? 2 : 0;
+    // ring depth / P buffers by update kind: the hi update usually stacks few rows (short K loops, the kernel
+    // streams P), the li update many.
+    const bool cfgB = slot == KT_DOWNDATE_HI;
+    const int S = cfgB ? 2 : 4, NX = cfgB ? 2 : 1;
+    // filters are processed in groups small enough for the per-CTA tile metadata (8 B per tile) to stay
+    // within the shared-memory budget of two CTAs per SM
+    const long long ctas_full = (long long)sms * 2;
+    const size_t fixed = sizeof(double) * (2 * S * TK * TPAD + NX * TM * XP) + sizeof(unsigned long long) * (2 * S + 2 * NX) +
+                         sizeof(unsigned) * T;
+    const size_t budget = 111 * 1024;
+    if (fixed + 64 * sizeof(int2) <= budget) {
+        const long long Mcap = (long long)((budget - fixed) / sizeof(int2));
+        long long bgroup = (Mcap * ctas_full) / T;
+        if (bgroup < 1) bgroup = 1;
+        const char* eg = getenv("EKFSLAM_DD_GROUP");   // =g: at most g filters per launch (exercises the grouping in tests)
+        const long long force_group = eg ? atoll(eg) : 0;
+        if (force_group > 0 && force_group < bgroup) bgroup = force_group;
+        for (long long b0 = 0; b0 < v.B; b0 += bgroup) {
+            const long long nb = (v.B - b0 < bgroup) ? (v.B - b0) : bgroup;
+            const long long total = (long long)T * nb;
+            const long long ctas = total < ctas_full ? total : ctas_full;
+            const int M = (int)((total + ctas - 1) / ctas);
+            const size_t sm2 = fixed + sizeof(int2) * M;
+            if (cfgB) ENSURE_DYN_SMEM((k_downdate_ws2<2, 2>), sm2, c->device);
+            else ENSURE_DYN_SMEM((k_downdate_ws2<4, 1>), sm2, c->device);
+            if (cfgB) k_downdate_ws2<2, 2><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
+            else k_downdate_ws2<4, 1><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
+            if (b0 > 0) c->launches++;
         }
-        const bool cfgB = cfgsel ? (cfgsel == 2) : (slot == KT_DOWNDATE_HI);
-        const int S = cfgB ? 2 : 4, NX = cfgB ? 2 : 1;
-        // filters are processed in groups small enough for the per-CTA tile metadata (8 B per tile) to stay
-        // within the shared-memory budget of two CTAs per SM
-        const long long ctas_full = (long long)sms * 2;
-        const int mirror = 1;   // P is kept exactly symmetric in memory: every off-diagonal tile is stored with its mirror image
-        const size_t fixed = sizeof(double) * (2 * S * TK * TPAD + NX * TM * XP) + sizeof(unsigned long long) * (2 * S + 2 * NX) +
-                             sizeof(unsigned) * T;
-        const size_t budget = 111 * 1024;
-        if (fixed + 64 * sizeof(int2) <= budget) {
-            const long long Mcap = (long long)((budget - fixed) / sizeof(int2));
-            long long bgroup = (Mcap * ctas_full) / T;
-            if (bgroup < 1) bgroup = 1;
-            const char* eg = getenv("EKFSLAM_DD_GROUP");   // =g: at most g filters per launch (exercises the grouping in tests)
-            const long long force_group = eg ? atoll(eg) : 0;
-            if (force_group > 0 && force_group < bgroup) bgroup = force_group;
-            for (long long b0 = 0; b0 < v.B; b0 += bgroup) {
-                const long long nb = (v.B - b0 < bgroup) ? (v.B - b0) : bgroup;
-                const long long total = (long long)T * nb;
-                const long long ctas = total < ctas_full ? total : ctas_full;
-                const int M = (int)((total + ctas - 1) / ctas);
-                const size_t sm2 = fixed + sizeof(int2) * M;
-                if (cfgB) ENSURE_DYN_SMEM((k_downdate_ws2<2, 2>), sm2, c->device);
-                else ENSURE_DYN_SMEM((k_downdate_ws2<4, 1>), sm2, c->device);
-                if (cfgB) k_downdate_ws2<2, 2><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M, mirror);
-                else k_downdate_ws2<4, 1><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M, mirror);
-                if (b0 > 0) c->launches++;
-            }
-            return;
-        }
+        return;
     }
+    // the tile table does not fit (li <4,1>: T > 2412, i.e. n_max > 4352; hi <2,2>: T > 2672, n_max > 4608): one CTA per tile
     const size_t sm = sizeof(double) * (2 * NSTAGE * TK * TPAD + TM * 9);
     ENSURE_DYN_SMEM(k_downdate_tile, sm, c->device);
     dim3 gd(T, v.B);

@@ -471,15 +471,13 @@ static size_t ransac_cluster_smem_bytes(const DevView& v) {
 }
 
 void launch_ransac(ekfslam_ctx* c) {
-    static int use_cluster = -1;
-    if (use_cluster < 0) { const char* e = getenv("EKFSLAM_RANSAC_CLUSTER"); use_cluster = (e && e[0] == '0') ? 0 : 1; }
     // fixed hypothesis budget (BASELINE configs 2 / 5: 256 / 512 draws): nearly every matched feature is drawn, so the
     // rows H P of the IC features come from one k_hp pass; adaptive rule (~7 scored hypotheses): built on demand
     const int prebuilt = c->prm.fixed_hyp > 0 ? 1 : 0;
     if (prebuilt) launch_hp(c, EKFSLAM_F_HAS_H | EKFSLAM_F_IC, 0);
     KScope ks(c, KT_RANSAC);
     // few filters + fixed hypothesis budget (the latency path): one cluster of CTAs per filter
-    if (use_cluster && c->prm.fixed_hyp > 0 && (long long)c->v.B * RANSAC_CLUSTER <= 2LL * c->sm_count) {
+    if (c->prm.fixed_hyp > 0 && (long long)c->v.B * RANSAC_CLUSTER <= 2LL * c->sm_count) {
         const size_t sm = ransac_cluster_smem_bytes(c->v);
         ENSURE_DYN_SMEM(k_ransac_fixed_cluster, sm, c->device);
         cudaLaunchConfig_t cfg = {};

@@ -11,8 +11,6 @@
 // Kernels: k_upd_S (select + stack S, nu) -> k_chol (blocked Cholesky, inv(L), y) ->
 //          k_gemm (W = inv(L) G_sel, triangular GEMM on DMMA; also x+, q normalisation, normJac) ->
 //          k_wfix (W <- W J', bookkeeping) -> k_downdate* (P <- J P J' - W'W, k_downdate.cu).
-#include <cstdlib>
-#include <cstring>
 #include "model.cuh"
 #include "tc_common.cuh"
 
@@ -395,7 +393,7 @@ __global__ void __launch_bounds__(128) k_chol(DevView v, int kskip) {
 // ---------------------------------------------------------------------------------------
 #define CHS_KL 200  // largest variant (a handful of filters per frame at N = 100): 144 < k <= 200, 512 threads, 190 KB -> 1 CTA/SM, own side stream
 #define CHS_K 144   // large variant: KMIN < k <= 144, 256 threads, 2 CTAs/SM
-#define CHS_KM 112  // middle variant (li update at N = 100: k ~ 100): 256 threads, <= 85 registers, 72 KB -> 3 CTAs/SM (EKFSLAM_CHOL_MID=0 disables)
+#define CHS_KM 112  // middle variant (li update at N = 100: k ~ 100): 256 threads, <= 85 registers, 72 KB -> 3 CTAs/SM
 #define CHS_KS 48   // small variant (hi update: k ~ 24): k <= 48, 128 threads, 21 KB of shared memory -> many CTAs/SM
 // Packed lower triangle whose rows start on an even index (16-byte aligned): the trailing update reads and writes four
 // neighbouring columns of a row as two 128-bit accesses.
@@ -1281,102 +1279,72 @@ void launch_update(ekfslam_ctx* c, int mask, int which_prior, int flags) {
     // 2.2 ms, lock-step 3.8 ms).  Few filters with a large stacked innovation (large maps): the single block is a
     // serial bottleneck (N=500, B=8: 7.1 of 11.5 ms per step), so every phase becomes its own launch over all
     // filters with the parallelism that phase has.
-    static int chol_mode = -1;
-    if (chol_mode < 0) {
-        const char* e = getenv("EKFSLAM_CHOL");
-        chol_mode = (e && !strcmp(e, "block")) ? 0 : (e && !strcmp(e, "lockstep")) ? 1 : 2;  // 2 = by shape
-    }
-    if (chol_mode == 1 || (chol_mode == 2 && v.B < 128 && v.kmax >= 256)) {
+    if (chol_lockstep(v)) {
         launch_chol_lockstep(c);
     } else {
         KScope ks(c, hi ? KT_CHOL_HI : KT_CHOL);
-        static int resident = -1;
-        if (resident < 0) {
-            const char* e = getenv("EKFSLAM_CHOL_SM");
-            resident = (e && e[0] == '0') ? 0 : 1;
-        }
-        if (resident) {
-            static int mid = -1;
-            if (mid < 0) { const char* e = getenv("EKFSLAM_CHOL_MID"); mid = (e && e[0] == '0') ? 0 : 1; }
-            const bool use_mid = mid && v.kmax > CHS_KM;
-            // 144 < k <= 200: the few filters of a frame with that many stacked rows used to go through k_chol (S in global
-            // memory, one 128-thread CTA each, ~0.28 ms of latency BEHIND the other variants); the resident kernel with 16
-            // warps takes them on a second side stream, under the main variant (EKFSLAM_CHOL_LARGE=0: the old path)
-            static int large_on = -1;
-            if (large_on < 0) { const char* e = getenv("EKFSLAM_CHOL_LARGE"); large_on = (e && e[0] == '0') ? 0 : 1; }
-            const bool large = large_on && use_mid && v.kmax > CHS_K;
-            auto fork_large = [&]() {   // after ev_fork has been recorded on st
-                if (!large) return;
+        const bool use_mid = v.kmax > CHS_KM;
+        // 144 < k <= 200: the few filters of a frame with that many stacked rows used to go through k_chol (S in global
+        // memory, one 128-thread CTA each, ~0.28 ms of latency BEHIND the other variants); the resident kernel with 16
+        // warps takes them on a second side stream, under the main variant
+        const bool large = use_mid && v.kmax > CHS_K;
+        auto fork_large = [&]() {   // after ev_fork has been recorded on st
+            if (!large) return;
+            cudaStreamWaitEvent(c->aux2_stream, c->ev_fork, 0);
+            k_chol_sm<CHS_KL, 512, CHS_K, 1><<<v.B, 512, chl_sm, c->aux2_stream>>>(v);
+            cudaEventRecord(c->ev_join2, c->aux2_stream);
+            c->launches++;
+        };
+        auto join_large = [&]() { if (large) cudaStreamWaitEvent(st, c->ev_join2, 0); };
+        if (hi) {   // few stacked rows are the rule: k <= 32, k <= CHS_KS, CHS_KS < k <= CHS_KM, and the rest
+            if (use_mid) {
+                // every variant is a chain of latencies that leaves the SMs mostly idle (one CTA per filter, a few hundred
+                // filters each): the warp-per-filter kernel (k <= 32) and the rarely used 144-row variant run on one side
+                // stream, the 48-row variant (and the 200-row one) on the other, the 112-row variant on the main stream -
+                // back to back they took 0.22 ms
+                cudaEventRecord(c->ev_fork, st);
+                cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0);
                 cudaStreamWaitEvent(c->aux2_stream, c->ev_fork, 0);
-                k_chol_sm<CHS_KL, 512, CHS_K, 1><<<v.B, 512, chl_sm, c->aux2_stream>>>(v);
+                k_chol_w32<<<(v.B + 3) / 4, 128, 0, c->aux_stream>>>(v);
+                k_chol_sm<CHS_K, 256, CHS_KM, 2><<<v.B, 256, chs_sm, c->aux_stream>>>(v);
+                cudaEventRecord(c->ev_join, c->aux_stream);
+                k_chol_sm<CHS_KS, 128, CHW_K><<<v.B, 128, chss_sm, c->aux2_stream>>>(v);
+                if (large) { k_chol_sm<CHS_KL, 512, CHS_K, 1><<<v.B, 512, chl_sm, c->aux2_stream>>>(v); c->launches++; }
                 cudaEventRecord(c->ev_join2, c->aux2_stream);
-                c->launches++;
-            };
-            auto join_large = [&]() { if (large) cudaStreamWaitEvent(st, c->ev_join2, 0); };
-            if (hi) {   // few stacked rows are the rule: k <= 32, k <= CHS_KS, CHS_KS < k <= CHS_KM, and the rest
-                static int w32 = -1;
-                if (w32 < 0) { const char* e = getenv("EKFSLAM_CHOL_W32"); w32 = (e && e[0] == '0') ? 0 : 1; }
-                if (use_mid) {
-                    // every variant is a chain of latencies that leaves the SMs mostly idle (one CTA per filter, a few hundred
-                    // filters each): the warp-per-filter kernel (k <= 32) and the rarely used 144-row variant run on one side
-                    // stream, the 48-row variant (and the 200-row one) on the other, the 112-row variant on the main stream -
-                    // back to back they took 0.22 ms
-                    cudaEventRecord(c->ev_fork, st);
-                    cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0);
-                    cudaStreamWaitEvent(c->aux2_stream, c->ev_fork, 0);
-                    if (w32) { k_chol_w32<<<(v.B + 3) / 4, 128, 0, c->aux_stream>>>(v); c->launches++; }
-                    k_chol_sm<CHS_K, 256, CHS_KM, 2><<<v.B, 256, chs_sm, c->aux_stream>>>(v);
-                    cudaEventRecord(c->ev_join, c->aux_stream);
-                    if (w32) k_chol_sm<CHS_KS, 128, CHW_K><<<v.B, 128, chss_sm, c->aux2_stream>>>(v);
-                    else k_chol_sm<CHS_KS, 128, 0><<<v.B, 128, chss_sm, c->aux2_stream>>>(v);
-                    if (large) { k_chol_sm<CHS_KL, 512, CHS_K, 1><<<v.B, 512, chl_sm, c->aux2_stream>>>(v); c->launches++; }
-                    cudaEventRecord(c->ev_join2, c->aux2_stream);
-                    k_chol_sm<CHS_KM, 256, CHS_KS, 3><<<v.B, 256, chsm_sm, st>>>(v);
-                    cudaStreamWaitEvent(st, c->ev_join, 0);
-                    cudaStreamWaitEvent(st, c->ev_join2, 0);
-                    c->launches += 2;
-                } else {
-                    if (w32) {   // k <= 32: a warp per filter, no block barriers; the 48-row variant keeps 32 < k <= 48
-                        k_chol_w32<<<(v.B + 3) / 4, 128, 0, st>>>(v);
-                        k_chol_sm<CHS_KS, 128, CHW_K><<<v.B, 128, chss_sm, st>>>(v);
-                        c->launches++;
-                    } else {
-                        k_chol_sm<CHS_KS, 128, 0><<<v.B, 128, chss_sm, st>>>(v);
-                    }
-                    k_chol_sm<CHS_K, 256, CHS_KS, 2><<<v.B, 256, chs_sm, st>>>(v);
-                    c->launches++;
-                }
+                k_chol_sm<CHS_KM, 256, CHS_KS, 3><<<v.B, 256, chsm_sm, st>>>(v);
+                cudaStreamWaitEvent(st, c->ev_join, 0);
+                cudaStreamWaitEvent(st, c->ev_join2, 0);
+                c->launches += 3;
             } else {
-                if (use_mid) {   // the common stacked sizes at 3 CTAs/SM, the rest in the large variant on the side stream
-                    cudaEventRecord(c->ev_fork, st);
-                    cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0);
-                    k_chol_sm<CHS_K, 256, CHS_KM, 2><<<v.B, 256, chs_sm, c->aux_stream>>>(v);
-                    cudaEventRecord(c->ev_join, c->aux_stream);
-                    fork_large();
-                    k_chol_sm<CHS_KM, 256, 0, 3><<<v.B, 256, chsm_sm, st>>>(v);
-                    cudaStreamWaitEvent(st, c->ev_join, 0);
-                    join_large();
-                    c->launches++;
-                } else {
-                    k_chol_sm<CHS_K, 256, 0, 2><<<v.B, 256, chs_sm, st>>>(v);
-                }
+                // k <= 32: a warp per filter, no block barriers; the 48-row variant keeps 32 < k <= 48
+                k_chol_w32<<<(v.B + 3) / 4, 128, 0, st>>>(v);
+                k_chol_sm<CHS_KS, 128, CHW_K><<<v.B, 128, chss_sm, st>>>(v);
+                k_chol_sm<CHS_K, 256, CHS_KS, 2><<<v.B, 256, chs_sm, st>>>(v);
+                c->launches += 2;
             }
-            const int kres = large ? CHS_KL : CHS_K;   // largest k the resident variants took
-            if (v.kmax > kres) { k_chol<<<v.B, 128, chol_sm, st>>>(v, kres); c->launches++; }
         } else {
-            k_chol<<<v.B, 128, chol_sm, st>>>(v, 0);
+            if (use_mid) {   // the common stacked sizes at 3 CTAs/SM, the rest in the large variant on the side stream
+                cudaEventRecord(c->ev_fork, st);
+                cudaStreamWaitEvent(c->aux_stream, c->ev_fork, 0);
+                k_chol_sm<CHS_K, 256, CHS_KM, 2><<<v.B, 256, chs_sm, c->aux_stream>>>(v);
+                cudaEventRecord(c->ev_join, c->aux_stream);
+                fork_large();
+                k_chol_sm<CHS_KM, 256, 0, 3><<<v.B, 256, chsm_sm, st>>>(v);
+                cudaStreamWaitEvent(st, c->ev_join, 0);
+                join_large();
+                c->launches++;
+            } else {
+                k_chol_sm<CHS_K, 256, 0, 2><<<v.B, 256, chs_sm, st>>>(v);
+            }
         }
+        const int kres = large ? CHS_KL : CHS_K;   // largest k the resident variants took
+        if (v.kmax > kres) { k_chol<<<v.B, 128, chol_sm, st>>>(v, kres); c->launches++; }
     }
     // (64-row tiles, column groups, filters): the li update has work in every filter -> long CTAs that walk all column
     // tiles; the hi update leaves few filters for this kernel (k_w_small takes k <= WS_K) -> two shorter CTAs per row tile
-    static int cg_li = -1, cg_hi = -1;
-    if (cg_li < 0) {
-        const char* e1 = getenv("EKFSLAM_W_CG_LI"); const char* e2 = getenv("EKFSLAM_W_CG_HI");
-        cg_li = e1 ? atoi(e1) : 1; cg_hi = e2 ? atoi(e2) : 2;   // hi: 2 / 3 / 5 / 10 column groups -> k_w_hi 0.43 / 0.44 / 0.47 / 0.56 ms
-        if (cg_li < 1) cg_li = 1; if (cg_hi < 1) cg_hi = 1;
-    }
+    // (hi: 2 / 3 / 5 / 10 column groups -> k_w_hi 0.43 / 0.44 / 0.47 / 0.56 ms)
+    int cg = hi ? 2 : 1;
     // few filters (large maps): split the column tiles so that the grid still fills the GPU
-    int cg = (mask & EKFSLAM_F_HI) ? cg_hi : cg_li;
     {
         const long long ctas = (long long)((v.kmax + TM - 1) / TM) * v.B;
         const int want = (int)((8LL * 148 + ctas - 1) / ctas);
@@ -1388,18 +1356,14 @@ void launch_update(ekfslam_ctx* c, int mask, int which_prior, int flags) {
     gemm_attr(c, w_sm);
     {
         KScope ks(c, hi ? KT_W_HI : KT_W);
-        static int small = -1;
-        if (small < 0) { const char* e = getenv("EKFSLAM_W_SMALL"); small = (e && e[0] == '0') ? 0 : 1; }
         const int fin = (flags & 2) ? 0 : 1;
-        if (small) {
-            const size_t ws_sm = sizeof(double) * 2 * WS_K * 128;
-            ENSURE_DYN_SMEM((k_w_small<WS_K, 0, 3>), ws_sm, c->device);
-            k_w_small<WS_K, 0, 3><<<v.B, 128, ws_sm, st>>>(v, fin);
-            c->launches++;
-        }
+        const size_t ws_sm = sizeof(double) * 2 * WS_K * 128;
+        ENSURE_DYN_SMEM((k_w_small<WS_K, 0, 3>), ws_sm, c->device);
+        k_w_small<WS_K, 0, 3><<<v.B, 128, ws_sm, st>>>(v, fin);
+        c->launches++;
         // (a persistent variant over a device-built list of the (filter, row tile) pairs with work was measured in round 2:
         // li 1.51 -> 1.67 ms, hi 0.58 -> 0.55 ms - the CTAs that find nothing to do are not what this launch costs)
-        k_gemm<0><<<gw, 256, w_sm, st>>>(v, fin, small ? WS_K : 0);
+        k_gemm<0><<<gw, 256, w_sm, st>>>(v, fin, WS_K);
     }
     if (flags & 2) return;   // not the last iterate of an iterated update: W is recomputed
     { KScope ks(c, KT_WFIX); k_wfix<<<v.B, 128, 0, st>>>(v); }

@@ -160,6 +160,19 @@ def test_large_map_n500(ekf):
     assert tot["li"] > 200
 
 
+def test_large_map_n724_tile_downdate(ekf):
+    """N=724 features (n=4357): the per-CTA tile table of the li downdate no longer fits the persistent kernel's shared
+    memory, so it falls back to one CTA per tile (k_downdate_tile), while the hi downdate stays on k_downdate_ws2 and the
+    Cholesky takes the lock-step blocked-64 path.  Same bar as N=500; the profiler confirms that the fallback ran."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        worst, tot = _run_sequence(ekf, B=1, N=724, frames=2, seed=710, n_u=64)
+    kernels = {e.name for e in prof.events()}
+    assert any("k_downdate_tile" in k for k in kernels), sorted(kernels)
+    assert any("k_downdate_ws2" in k for k in kernels), sorted(kernels)
+    assert tot["li"] > 200
+
+
 def test_ragged_batch_and_unpredicted_features(ekf):
     """Filters of one batch with different map sizes (24, 17, 5 and 0 features: n = 157, 115, 43, 13) and features that
     are never predicted (ray pointing away from the camera: h / H / S stay empty, mc/predict_camera_measurements.m:14-16)."""
@@ -192,16 +205,12 @@ def test_n120_more_than_200_stacked_rows(ekf):
     assert tot["li"] > 2 * 2 * 100, tot
 
 
-def test_row_pitch_knob(ekf, monkeypatch):
-    """Row pitch of x / P / G: 256 bytes by default (ld % 32 == 0), EKFSLAM_LD_ALIGN restores the minimal pitch; the partial last
-    tile column of the covariance downdate differs between the two (n = 85: ld 96 vs 88), results must not."""
+def test_row_pitch_256_bytes(ekf):
+    """Row pitch of x / P / G: a multiple of 256 bytes (ld % 32 == 0); at n = 85 (ld = 96) the last 64-wide tile column of the
+    covariance downdate is partial, results must not differ from the oracle."""
     pkg, _ = ekf
     bank = pkg.FilterBank(1, 12, 85)
     assert bank.ld % 32 == 0 and bank.ld >= 85
-    bank.close()
-    monkeypatch.setenv("EKFSLAM_LD_ALIGN", "8")
-    bank = pkg.FilterBank(1, 12, 85)
-    assert bank.ld == 88
     bank.close()
     worst, tot = _run_sequence(ekf, B=3, N=12, frames=3, seed=860)
     assert tot["li"] > 30, tot
