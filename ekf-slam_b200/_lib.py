@@ -44,6 +44,17 @@ class Stats(C.Structure):
 STATS_FIELDS = [f[0] for f in Stats._fields_]
 
 
+class Eval(C.Structure):
+    _fields_ = [("pos_sq_err", C.c_double), ("rot_sq_err", C.c_double), ("nees_pos", C.c_double),
+                ("nees_pose", C.c_double), ("map_sq_err", C.c_double), ("map_nees", C.c_double),
+                ("n_map", C.c_int32), ("n_skip", C.c_int32), ("frames", C.c_int32), ("status", C.c_int32)]
+
+
+EVAL_FIELDS = [f[0] for f in Eval._fields_]
+# ekfslam_eval.status bits
+EVAL_CAM_NOT_SPD, EVAL_NO_TRUTH, EVAL_NOT_EVALUABLE = 1, 2, 4
+
+
 class WorldParams(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("b_offset", C.c_int32), ("flaky_mod", C.c_int32), ("noise_px", C.c_double),
                 ("gross_px", C.c_double), ("p_outlier", C.c_double), ("p_flaky", C.c_double), ("band_px", C.c_double)]
@@ -108,6 +119,10 @@ _SIGS = {
     "ekfslam_world_detect": (_I, [_P, _I, _I]),
     "ekfslam_world_uniforms": (_I, [_P, _I, _I]),
     "ekfslam_download_uniforms": (_I, [_P, _I, _I, _P, _I]),
+    "ekfslam_evaluate": (_I, [_P, _I]),
+    "ekfslam_download_eval": (_I, [_P, _I, _I, _I, _P, _P, _P]),
+    "ekfslam_reset_eval": (_I, [_P]),
+    "ekfslam_map_cartesian": (_I, [_P, _I, _I, _P, _P]),
     "ekfslam_device_ptr": (_P, [_P, C.c_char_p]),
     "ekfslam_enable_timing": (_I, [_P, _I]),
     "ekfslam_kernel_count": (_I, []),

@@ -316,6 +316,46 @@ class FilterBank:
     def world_detect(self, t, K):
         L.check(self.lib.ekfslam_world_detect(self._h, int(t), int(K)))
 
+    # -- scoring against the resident ground truth ------------------------------------------------
+    def evaluate(self, t):
+        """Scores every filter's (x_k_k, P) against frame t of the uploaded world (see ekfslam_evaluate): the frame's
+        record replaces the last one and is added into the running totals.  Stream-ordered, no host copies."""
+        L.check(self.lib.ekfslam_evaluate(self._h, int(t)))
+
+    def download_eval(self, totals=False, b0=0, nb=None, features=True):
+        """{field: [nb] array} of the last frame's records (totals=False) or of the running totals (totals=True);
+        float64 for the error / NEES sums, int32 for n_map, n_skip, frames, status.  With totals=False and
+        features=True also feat_err [nb, N, 3] and feat_nees [nb, N] (NaN where a slot is empty, has no truth or is
+        not evaluable)."""
+        nb = self.B - b0 if nb is None else nb
+        rec = (L.Eval * nb)()
+        fe = fn = None
+        if features and not totals:
+            fe, fn = np.empty((nb, self.N, 3)), np.empty((nb, self.N))
+        L.check(self.lib.ekfslam_download_eval(self._h, b0, nb, 1 if totals else 0, C.cast(rec, C.c_void_p),
+                                               _ptr(fe), _ptr(fn)))
+        out = {k: np.array([getattr(r, k) for r in rec], dtype=np.float64 if i < 6 else np.int32)
+               for i, k in enumerate(L.EVAL_FIELDS)}
+        if fe is not None:
+            out["feat_err"], out["feat_nees"] = fe, fn
+        return out
+
+    def reset_eval(self):
+        """Zeroes the running totals."""
+        L.check(self.lib.ekfslam_reset_eval(self._h))
+
+    def map_cartesian(self, b0=0, nb=None):
+        """The maps in Cartesian coordinates: p [nb, N, 3] and C [nb, N, 3, 3] (NaN for empty and not evaluable
+        slots).  Needs no world."""
+        nb = self.B - b0 if nb is None else nb
+        p, packed = np.empty((nb, self.N, 3)), np.empty((nb, self.N, 6))
+        L.check(self.lib.ekfslam_map_cartesian(self._h, b0, nb, _ptr(p), _ptr(packed)))
+        C3 = np.empty((nb, self.N, 3, 3))
+        for k, (i, j) in enumerate(((0, 0), (1, 0), (1, 1), (2, 0), (2, 1), (2, 2))):
+            C3[..., i, j] = packed[..., k]
+            C3[..., j, i] = packed[..., k]
+        return p, C3
+
     # -- stages (names follow the reference functions they replace) --------------------------
     def begin_frame(self):
         L.check(self.lib.ekfslam_begin_frame(self._h))

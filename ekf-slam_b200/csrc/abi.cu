@@ -98,7 +98,7 @@ static void kt_collect(ekfslam_ctx* c) {
 static const char* KT_NAMES[KT_COUNT] = {"k_begin_frame", "k_predict", "k_features", "k_hp", "k_innov", "k_ransac",
                                          "k_upd_S", "k_chol", "k_w", "k_downdate_hi", "k_downdate", "k_symmetrize",
                                          "k_add_features", "k_wfix", "k_w_hi", "k_chol_hi", "k_upd_S_hi",
-                                         "k_hp_rescue", "k_world"};
+                                         "k_hp_rescue", "k_world", "k_eval"};
 
 template <typename T>
 static cudaError_t dalloc(T** p, size_t count, int64_t* total) {
@@ -279,7 +279,8 @@ int ekfslam_destroy(ekfslam_ctx* c) {
     DevView& v = c->v;
     void* ptrs[] = {v.x, v.xp, v.P, v.G, v.W, v.Sb, v.Li, v.yv, v.jn, v.jnt, v.ktot, v.kmaxdev, v.cv, v.h, v.Hc, v.S, v.z, v.zc, v.u, v.ftype,
                     v.flags, v.mflags, v.foff, v.nstate, v.nfeat, v.counters, v.tag, v.sel, v.ksel, v.stats, v.nhyp_tab,
-                    c->mm_del, c->mm_quota, c->det_n, c->det_uv, c->det_tag, c->world_points, c->world_poses};
+                    c->mm_del, c->mm_quota, c->det_n, c->det_uv, c->det_tag, c->world_points, c->world_poses,
+                    c->ev.rec, c->ev.tot, c->ev.ferr, c->ev.fnees, c->ev.mp, c->ev.mc};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (c->timer) {
@@ -1095,6 +1096,89 @@ int ekfslam_world_detect(ekfslam_ctx* c, int t, int K) {
     if (int r = ensure_det(c, K)) return r;
     launch_world_detect(c, t);
     LAUNCHED();
+    return EKFSLAM_OK;
+}
+
+// ---- scoring against the resident ground truth (k_eval.cu) -------------------------------------
+// shared memory of the scoring launch: two doubles and one byte per feature slot
+static int eval_fits(const ekfslam_ctx* c) {
+    if ((size_t)c->v.N * 17 > 200 * 1024) return fail(EKFSLAM_ERR_INVALID, "evaluation supports N_max <= 12000");
+    return EKFSLAM_OK;
+}
+
+int ekfslam_evaluate(ekfslam_ctx* c, int t) {
+    NEED_CTX(c);
+    if (!c->world_points) return fail(EKFSLAM_ERR_STATE, "evaluate: no world uploaded (ekfslam_world_upload)");
+    if (t < 0 || t > c->world.T) return fail(EKFSLAM_ERR_INVALID, "frame index out of [0, T]");
+    if (int r = eval_fits(c)) return r;
+    DevEval& e = c->ev;
+    if (!e.rec) {   // first evaluation: the buffers are allocated here, so a context that never evaluates holds none
+        const size_t B = (size_t)c->v.B, BN = B * c->v.N;
+        cudaError_t er = cudaMalloc((void**)&e.rec, sizeof(ekfslam_eval) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&e.tot, sizeof(ekfslam_eval) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&e.ferr, sizeof(double) * 3 * BN);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&e.fnees, sizeof(double) * BN);
+        if (er != cudaSuccess) {   // all or nothing: e.rec != null means every scoring buffer exists
+            for (void* q : {(void*)e.rec, (void*)e.tot, (void*)e.ferr, (void*)e.fnees}) if (q) cudaFree(q);
+            e.rec = e.tot = nullptr; e.ferr = e.fnees = nullptr;
+            cudaGetLastError();   // an allocation failure is reported here, not by the next launch check
+            return fail(er == cudaErrorMemoryAllocation ? EKFSLAM_ERR_NOMEM : EKFSLAM_ERR_CUDA,
+                        std::string("evaluation buffers: ") + cudaGetErrorString(er));
+        }
+        CK(cudaMemsetAsync(e.tot, 0, sizeof(ekfslam_eval) * B, c->stream));
+        c->bytes += (int64_t)(2 * sizeof(ekfslam_eval) * B + sizeof(double) * 4 * BN);
+    }
+    launch_eval(c, 0, t, 0, c->v.B);
+    LAUNCHED();
+    return EKFSLAM_OK;
+}
+
+int ekfslam_download_eval(ekfslam_ctx* c, int b0, int nb, int totals, ekfslam_eval* rec, double* feat_err,
+                          double* feat_nees) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    if (!rec) return fail(EKFSLAM_ERR_INVALID, "rec is null");
+    if (totals && (feat_err || feat_nees))
+        return fail(EKFSLAM_ERR_INVALID, "per-feature outputs exist for the last frame only (totals == 0)");
+    const DevEval& e = c->ev;
+    if (!e.rec) return fail(EKFSLAM_ERR_STATE, "nothing evaluated yet (ekfslam_evaluate)");
+    const size_t o = (size_t)b0 * c->v.N, cnt = (size_t)nb * c->v.N;
+    CK(cudaMemcpyAsync(rec, (totals ? e.tot : e.rec) + b0, sizeof(ekfslam_eval) * nb, cudaMemcpyDeviceToHost, c->stream));
+    if (feat_err) CK(cudaMemcpyAsync(feat_err, e.ferr + 3 * o, sizeof(double) * 3 * cnt, cudaMemcpyDeviceToHost, c->stream));
+    if (feat_nees) CK(cudaMemcpyAsync(feat_nees, e.fnees + o, sizeof(double) * cnt, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return EKFSLAM_OK;
+}
+
+int ekfslam_reset_eval(ekfslam_ctx* c) {
+    NEED_CTX(c);
+    if (c->ev.tot) CK(cudaMemsetAsync(c->ev.tot, 0, sizeof(ekfslam_eval) * c->v.B, c->stream));
+    return EKFSLAM_OK;
+}
+
+int ekfslam_map_cartesian(ekfslam_ctx* c, int b0, int nb, double* p, double* cov) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    DevEval& e = c->ev;
+    const size_t BN = (size_t)c->v.B * c->v.N;
+    if (!e.mp) {
+        cudaError_t er = cudaMalloc((void**)&e.mp, sizeof(double) * 3 * BN);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&e.mc, sizeof(double) * 6 * BN);
+        if (er != cudaSuccess) {
+            if (e.mp) cudaFree(e.mp);
+            e.mp = nullptr;
+            cudaGetLastError();
+            return fail(er == cudaErrorMemoryAllocation ? EKFSLAM_ERR_NOMEM : EKFSLAM_ERR_CUDA,
+                        std::string("map export buffers: ") + cudaGetErrorString(er));
+        }
+        c->bytes += (int64_t)(sizeof(double) * 9 * BN);
+    }
+    launch_eval(c, 1, 0, b0, nb);
+    LAUNCHED();
+    const size_t o = (size_t)b0 * c->v.N, cnt = (size_t)nb * c->v.N;
+    if (p) CK(cudaMemcpyAsync(p, e.mp + 3 * o, sizeof(double) * 3 * cnt, cudaMemcpyDeviceToHost, c->stream));
+    if (cov) CK(cudaMemcpyAsync(cov, e.mc + 6 * o, sizeof(double) * 6 * cnt, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
     return EKFSLAM_OK;
 }
 

@@ -70,9 +70,20 @@ struct DevWorld {
 // per-kernel timing (ekfslam_enable_timing): every launch is bracketed by an event pair
 enum {
     KT_BEGIN_FRAME = 0, KT_PREDICT, KT_FEATURES, KT_HP, KT_INNOV, KT_RANSAC, KT_UPD_S, KT_CHOL, KT_W, KT_DOWNDATE_HI,
-    KT_DOWNDATE, KT_SYMMETRIZE, KT_ADD_FEATURES, KT_WFIX, KT_W_HI, KT_CHOL_HI, KT_UPD_S_HI, KT_HP_RESCUE, KT_WORLD, KT_COUNT
+    KT_DOWNDATE, KT_SYMMETRIZE, KT_ADD_FEATURES, KT_WFIX, KT_W_HI, KT_CHOL_HI, KT_UPD_S_HI, KT_HP_RESCUE, KT_WORLD, KT_EVAL, KT_COUNT
 };
 struct KTimer;
+
+// scoring against the resident ground truth (k_eval.cu); allocated on the first ekfslam_evaluate /
+// ekfslam_map_cartesian, so a context that never evaluates holds none of it
+struct DevEval {
+    ekfslam_eval* rec;    // [B]        record of the last evaluated frame
+    ekfslam_eval* tot;    // [B]        running totals
+    double* ferr;         // [B][N][3]  e_f of the last evaluated frame
+    double* fnees;        // [B][N]     nees_f of the last evaluated frame
+    double* mp;           // [B][N][3]  map export: p
+    double* mc;           // [B][N][6]  map export: C_f packed (xx, yx, yy, zx, zy, zz)
+};
 
 struct ekfslam_ctx {
     int device;
@@ -110,6 +121,7 @@ struct ekfslam_ctx {
     uint8_t* mm_del; int32_t* mm_quota;                             // [B][N], [B]
     // the context's own frame buffers while caller-owned ones are bound (ekfslam_bind_frame)
     double* own_zc; uint8_t* own_mflags; double* own_u; int own_n_u;
+    DevEval ev;
 };
 
 // W is stored panel-major: element (row t, column c) of a filter lives at ((c / 64) * wrows + t) * EKF_WPAD + c % 64.
@@ -179,3 +191,5 @@ void launch_world_candidates(ekfslam_ctx* c, int t);
 void launch_world_detect(ekfslam_ctx* c, int t);
 void launch_world_uniforms(ekfslam_ctx* c, int t);
 void launch_mm_plan(ekfslam_ctx* c, int min_features);
+// mode 0: score filters [b0, b0+nb) against frame t of the world; mode 1: map export of filters [b0, b0+nb)
+void launch_eval(ekfslam_ctx* c, int mode, int t, int b0, int nb);

@@ -223,6 +223,7 @@ class SynthSequence:
     def __init__(self, B, N, T, seed=0, b_offset=0, p_outlier=0.2, noise_px=0.5, cam=None,
                  depth_range=(2.0, 10.0), margin_px=45.0, n_u=64):
         self.B, self.N, self.T, self.n_u = B, N, T, n_u
+        self.seed, self.b_offset, self.p_outlier, self.noise_px = int(seed), int(b_offset), float(p_outlier), float(noise_px)
         self.cam = cam or default_camera()
         cam = self.cam
         T1 = T + 1
@@ -296,6 +297,15 @@ class SynthSequence:
             Pxv[:, i, i] = 0.025 ** 2
         x, P = initial_map(xv, Pxv, self.zc[0, b0:b0 + nb], self.cam, std_pxl=std_pxl)
         return x, P, np.ones((nb, self.N), dtype=np.uint8)
+
+    def truth_world(self):
+        """The sequence's own ground truth as a world for ``FilterBank.world_upload``: M = N points (world point k is
+        feature k, so ``upload_feature_meta(tag=arange(N))`` lets ``FilterBank.evaluate`` score the filters) and the
+        T+1 true poses.  Candidates the device world draws from it follow this sequence's noise model (pixel noise,
+        U(-8, 8) gross outliers with probability p_outlier), not its draws."""
+        return SimpleNamespace(points=self.points, pose_r=self.pose_r, pose_q=self.pose_q, M=self.N, T=self.T,
+                               seed=self.seed, b_offset=self.b_offset, flaky_mod=1, noise_px=self.noise_px,
+                               gross_px=8.0, p_outlier=self.p_outlier, p_flaky=self.p_outlier, BAND=SynthWorld.BAND)
 
     def frame(self, t):
         """Candidates of frame t (1..T): zc [B,N,2], has [B,N] u8."""

@@ -303,6 +303,52 @@ int ekfslam_world_uniforms(ekfslam_ctx* ctx, int t, int n_u);
 /* the resident uniform stream, u [nb][n_u] (n_u must equal the resident stream's length) */
 int ekfslam_download_uniforms(ekfslam_ctx* ctx, int b0, int nb, double* u, int n_u);
 
+/* ---- scoring against the resident ground truth (B independent Monte-Carlo runs) ---- */
+/* Evaluation reads the resident estimate (x_k_k, P): called between ekfslam_predict and the li update it scores the
+ * predicted covariance.  It touches nothing else of the filter (x, xp, P, flags, counters, tags and stats are
+ * read-only to it).  Definitions, with (r_t, q_t) the true pose of frame t (q scalar first):
+ *   camera:  e_r = x[0:3] - r_t;  d = conj(q_t) * x[3:7] (not renormalised), s = sign(d_w) (+1 at 0),
+ *            e_theta = 2 s d_xyz, angle = 2 atan2(|d_xyz|, |d_w|);  J = blockdiag(I3, 2 s E Q_L(conj(q_t))) on the 7
+ *            (r, q) columns (Q_L = left-multiplication matrix, E keeps rows 1..3), C_pose = J P[0:7,0:7] J' (6x6);
+ *            nees_pos = e_r' inv(P_rr) e_r (3 dof), nees_pose = e' inv(C_pose) e with e = [e_r; e_theta] (6 dof),
+ *            both through a Cholesky factorisation.
+ *   feature: slot i of filter b is valid when i < nfeat[b]; its tag names its world point.  Inverse-depth
+ *            [x y z theta phi rho] -> p = [x y z] + m(theta, phi) / rho, m = [cos(phi) sin(theta), -sin(phi),
+ *            cos(phi) cos(theta)] (mc/inversedepth_2_cartesian.m:37-45), a Cartesian block is p itself;
+ *            C_f = J_f P_ff J_f' (3x3), e_f = p - points[b][tag], nees_f = e_f' inv(C_f) e_f (Cholesky).
+ *            rho <= 0 or a Cholesky pivot of C_f <= 0: not evaluable (NaN per-feature outputs, n_skip, status bit 2);
+ *            a tag outside [0, M): no truth (NaN, n_skip, status bit 1).
+ * Sums run over the evaluable features in feature order; the reduction has a fixed order (no floating-point
+ * atomics), so a record is bit-identical from run to run.  When a camera Cholesky pivot is <= 0 the affected NEES
+ * (nees_pose, and nees_pos when P_rr itself fails) is NaN and status bit 0 is set; a NaN carries into the totals. */
+typedef struct {
+    double pos_sq_err;  /* |e_r|^2                                   */
+    double rot_sq_err;  /* angle^2 [rad^2]                           */
+    double nees_pos;    /* 3 dof                                     */
+    double nees_pose;   /* 6 dof                                     */
+    double map_sq_err;  /* sum of |e_f|^2 over the evaluable features */
+    double map_nees;    /* sum of nees_f over the evaluable features  */
+    int32_t n_map;      /* evaluable features                        */
+    int32_t n_skip;     /* valid slots without truth or not evaluable */
+    int32_t frames;     /* 1 per evaluation (totals: frames summed)  */
+    int32_t status;     /* bit0: camera covariance not SPD; bit1: a feature without truth; bit2: a feature not evaluable */
+} ekfslam_eval;
+/* score every filter against frame t of the world (ekfslam_world_upload); stream-ordered, no host copies.  The
+ * per-frame record replaces the previous one and is added field by field (status OR-ed) into the running totals.
+ * ERR_STATE without a world, ERR_INVALID for t outside [0, T]. */
+int ekfslam_evaluate(ekfslam_ctx* ctx, int t);
+/* rec [nb]: the last frame's records (totals == 0) or the running totals (totals != 0).  feat_err [nb][N_max][3] and
+ * feat_nees [nb][N_max] (either may be NULL) are the last frame's e_f and nees_f, NaN where a slot is empty, has no
+ * truth or is not evaluable; they exist only for the last frame, so they must be NULL when totals != 0.
+ * ERR_STATE before the first ekfslam_evaluate. */
+int ekfslam_download_eval(ekfslam_ctx* ctx, int b0, int nb, int totals, ekfslam_eval* rec, double* feat_err,
+                          double* feat_nees);
+/* zero the running totals (stream-ordered) */
+int ekfslam_reset_eval(ekfslam_ctx* ctx);
+/* the map in Cartesian coordinates, no world needed: p [nb][N_max][3] = p of every slot, cov [nb][N_max][6] = C_f
+ * packed (xx, yx, yy, zx, zy, zz); NaN for empty and not evaluable slots.  Either pointer may be NULL. */
+int ekfslam_map_cartesian(ekfslam_ctx* ctx, int b0, int nb, double* p, double* cov);
+
 /* ---- measurement hooks ------------------------------------------------------ */
 /* bracket every kernel launch with a CUDA event pair on the context's stream and accumulate the
  * elapsed time per kernel; enabling again resets the accumulators, on=0 removes the events */
