@@ -53,6 +53,8 @@ class Eval(C.Structure):
 EVAL_FIELDS = [f[0] for f in Eval._fields_]
 # ekfslam_eval.status bits
 EVAL_CAM_NOT_SPD, EVAL_NO_TRUTH, EVAL_NOT_EVALUABLE = 1, 2, 4
+# per-filter status of ekfslam_update_camera
+CAM_APPLIED, CAM_OFF, CAM_GATED, CAM_NOT_SPD = 0, 1, 2, 3
 
 
 class WorldParams(C.Structure):
@@ -123,6 +125,8 @@ _SIGS = {
     "ekfslam_download_eval": (_I, [_P, _I, _I, _I, _P, _P, _P]),
     "ekfslam_reset_eval": (_I, [_P]),
     "ekfslam_map_cartesian": (_I, [_P, _I, _I, _P, _P]),
+    "ekfslam_update_camera": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, C.c_double, _I]),
+    "ekfslam_download_camera_update": (_I, [_P, _I, _I, _P, _P]),
     "ekfslam_device_ptr": (_P, [_P, C.c_char_p]),
     "ekfslam_enable_timing": (_I, [_P, _I]),
     "ekfslam_kernel_count": (_I, []),

@@ -356,6 +356,36 @@ class FilterBank:
             C3[..., j, i] = packed[..., k]
         return p, C3
 
+    # -- camera-state measurement update (extension) ---------------------------------------------
+    def update_camera(self, H, z, R, on=None, gate=0.0, which=0, b0=0):
+        """Linear update of the camera state x[0:13] with m rows z = H x[0:13] + v, v ~ N(0, R), per filter (see
+        ekfslam_update_camera).  H [m,13] and R [m,m] are shared by every filter, [nb,m,13] and [nb,m,m] are taken per
+        filter; z [nb,m]; on [nb] (None = all).  which=0 updates (x_k_k, P), which=1 (x_k_km1, P); gate <= 0: no
+        chi-square gate.  Stream-ordered; the per-filter NIS and status come from download_camera_update()."""
+        z = _c(z, np.float64)
+        if z.ndim != 2:
+            raise ValueError("z must be [nb, m]")
+        nb, m = z.shape
+        H = np.asarray(H, dtype=np.float64)
+        R = np.asarray(R, dtype=np.float64)
+        if H.shape == (m, 13):
+            H = np.broadcast_to(H, (nb, m, 13))
+        if R.shape == (m, m):
+            R = np.broadcast_to(R, (nb, m, m))
+        H = _c(H, np.float64, (nb, m, 13))
+        R = _c(R, np.float64, (nb, m, m))
+        on = None if on is None else _c(on, np.uint8, (nb,))
+        L.check(self.lib.ekfslam_update_camera(self._h, int(b0), nb, m, _ptr(H), _ptr(z), _ptr(R), _ptr(on),
+                                               float(gate), int(which)))
+
+    def download_camera_update(self, b0=0, nb=None):
+        """{"nis": float64 [nb], "status": int32 [nb]} of the last update_camera (status: CAM_APPLIED, CAM_OFF,
+        CAM_GATED, CAM_NOT_SPD; NIS is NaN for CAM_OFF and CAM_NOT_SPD)."""
+        nb = self.B - b0 if nb is None else nb
+        nis, st = np.empty(nb), np.empty(nb, dtype=np.int32)
+        L.check(self.lib.ekfslam_download_camera_update(self._h, b0, nb, _ptr(nis), _ptr(st)))
+        return {"nis": nis, "status": st}
+
     # -- stages (names follow the reference functions they replace) --------------------------
     def begin_frame(self):
         L.check(self.lib.ekfslam_begin_frame(self._h))

@@ -98,7 +98,7 @@ static void kt_collect(ekfslam_ctx* c) {
 static const char* KT_NAMES[KT_COUNT] = {"k_begin_frame", "k_predict", "k_features", "k_hp", "k_innov", "k_ransac",
                                          "k_upd_S", "k_chol", "k_w", "k_downdate_hi", "k_downdate", "k_symmetrize",
                                          "k_add_features", "k_wfix", "k_w_hi", "k_chol_hi", "k_upd_S_hi",
-                                         "k_hp_rescue", "k_world", "k_eval"};
+                                         "k_hp_rescue", "k_world", "k_eval", "k_cam_update", "k_downdate_cam"};
 
 template <typename T>
 static cudaError_t dalloc(T** p, size_t count, int64_t* total) {
@@ -280,7 +280,8 @@ int ekfslam_destroy(ekfslam_ctx* c) {
     void* ptrs[] = {v.x, v.xp, v.P, v.G, v.W, v.Sb, v.Li, v.yv, v.jn, v.jnt, v.ktot, v.kmaxdev, v.cv, v.h, v.Hc, v.S, v.z, v.zc, v.u, v.ftype,
                     v.flags, v.mflags, v.foff, v.nstate, v.nfeat, v.counters, v.tag, v.sel, v.ksel, v.stats, v.nhyp_tab,
                     c->mm_del, c->mm_quota, c->det_n, c->det_uv, c->det_tag, c->world_points, c->world_poses,
-                    c->ev.rec, c->ev.tot, c->ev.ferr, c->ev.fnees, c->ev.mp, c->ev.mc};
+                    c->ev.rec, c->ev.tot, c->ev.ferr, c->ev.fnees, c->ev.mp, c->ev.mc,
+                    c->cu.H, c->cu.z, c->cu.R, c->cu.on, c->cu.nis, c->cu.status};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (c->timer) {
@@ -1178,6 +1179,57 @@ int ekfslam_map_cartesian(ekfslam_ctx* c, int b0, int nb, double* p, double* cov
     const size_t o = (size_t)b0 * c->v.N, cnt = (size_t)nb * c->v.N;
     if (p) CK(cudaMemcpyAsync(p, e.mp + 3 * o, sizeof(double) * 3 * cnt, cudaMemcpyDeviceToHost, c->stream));
     if (cov) CK(cudaMemcpyAsync(cov, e.mc + 6 * o, sizeof(double) * 6 * cnt, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return EKFSLAM_OK;
+}
+
+// ---- camera-state measurement update (k_cam_update.cu) ------------------------------------------
+int ekfslam_update_camera(ekfslam_ctx* c, int b0, int nb, int m, const double* H, const double* z, const double* R,
+                          const uint8_t* on, double gate, int which) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    const int mmax = c->v.kmax < EKF_XV ? c->v.kmax : EKF_XV;   // W has 2 N_max rows per panel
+    if (m < 1 || m > mmax) return fail(EKFSLAM_ERR_INVALID, "m must be in [1, min(13, 2 N_max)]");
+    if (which != 0 && which != 1) return fail(EKFSLAM_ERR_INVALID, "which must be 0 (x_k_k) or 1 (x_k_km1)");
+    if (!H || !z || !R) return fail(EKFSLAM_ERR_INVALID, "H / z / R is null");
+    DevCamUpd& u = c->cu;
+    const size_t B = (size_t)c->v.B;
+    if (!u.H) {   // first call: the buffers are allocated here, so a context that never calls this holds none
+        const size_t mm = (size_t)EKF_XV * EKF_XV;
+        cudaError_t er = cudaMalloc((void**)&u.H, sizeof(double) * mm * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.z, sizeof(double) * EKF_XV * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.R, sizeof(double) * mm * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.on, B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.nis, sizeof(double) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.status, sizeof(int32_t) * B);
+        if (er != cudaSuccess) {   // all or nothing: u.H != null means every staging buffer exists
+            for (void* q : {(void*)u.H, (void*)u.z, (void*)u.R, (void*)u.on, (void*)u.nis, (void*)u.status}) if (q) cudaFree(q);
+            u = DevCamUpd();
+            cudaGetLastError();
+            return fail(er == cudaErrorMemoryAllocation ? EKFSLAM_ERR_NOMEM : EKFSLAM_ERR_CUDA,
+                        std::string("camera update buffers: ") + cudaGetErrorString(er));
+        }
+        c->bytes += (int64_t)((sizeof(double) * (2 * mm + EKF_XV + 1) + 1 + sizeof(int32_t)) * B);
+    }
+    u.m = m; u.b0 = b0; u.nb = nb; u.gate = gate;
+    const size_t n = (size_t)nb;
+    CK(cudaMemcpyAsync(u.H + (size_t)b0 * m * EKF_XV, H, sizeof(double) * n * m * EKF_XV, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(u.z + (size_t)b0 * m, z, sizeof(double) * n * m, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(u.R + (size_t)b0 * m * m, R, sizeof(double) * n * m * m, cudaMemcpyHostToDevice, c->stream));
+    if (on) CK(cudaMemcpyAsync(u.on + b0, on, n, cudaMemcpyHostToDevice, c->stream));
+    else CK(cudaMemsetAsync(u.on + b0, 1, n, c->stream));
+    launch_cam_update(c, which);
+    LAUNCHED();
+    return EKFSLAM_OK;
+}
+
+int ekfslam_download_camera_update(ekfslam_ctx* c, int b0, int nb, double* nis, int32_t* status) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    const DevCamUpd& u = c->cu;
+    if (!u.H) return fail(EKFSLAM_ERR_STATE, "no camera update yet (ekfslam_update_camera)");
+    if (nis) CK(cudaMemcpyAsync(nis, u.nis + b0, sizeof(double) * nb, cudaMemcpyDeviceToHost, c->stream));
+    if (status) CK(cudaMemcpyAsync(status, u.status + b0, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     return EKFSLAM_OK;
 }

@@ -70,7 +70,8 @@ struct DevWorld {
 // per-kernel timing (ekfslam_enable_timing): every launch is bracketed by an event pair
 enum {
     KT_BEGIN_FRAME = 0, KT_PREDICT, KT_FEATURES, KT_HP, KT_INNOV, KT_RANSAC, KT_UPD_S, KT_CHOL, KT_W, KT_DOWNDATE_HI,
-    KT_DOWNDATE, KT_SYMMETRIZE, KT_ADD_FEATURES, KT_WFIX, KT_W_HI, KT_CHOL_HI, KT_UPD_S_HI, KT_HP_RESCUE, KT_WORLD, KT_EVAL, KT_COUNT
+    KT_DOWNDATE, KT_SYMMETRIZE, KT_ADD_FEATURES, KT_WFIX, KT_W_HI, KT_CHOL_HI, KT_UPD_S_HI, KT_HP_RESCUE, KT_WORLD, KT_EVAL,
+    KT_CAM_UPDATE, KT_DOWNDATE_CAM, KT_COUNT
 };
 struct KTimer;
 
@@ -83,6 +84,19 @@ struct DevEval {
     double* fnees;        // [B][N]     nees_f of the last evaluated frame
     double* mp;           // [B][N][3]  map export: p
     double* mc;           // [B][N][6]  map export: C_f packed (xx, yx, yy, zx, zy, zz)
+};
+
+// camera-state measurement update (k_cam_update.cu); allocated on the first ekfslam_update_camera, so a context that
+// never calls it holds none of it.  H, z and R are packed with the m of the last call.
+struct DevCamUpd {
+    double* H;            // [B][m][13]
+    double* z;            // [B][m]
+    double* R;            // [B][m][m]  (lower triangle read)
+    uint8_t* on;          // [B]
+    double* nis;          // [B]
+    int32_t* status;      // [B]        EKFSLAM_CAM_*
+    int m, b0, nb;        // rows and filter range of the last call
+    double gate;          // <= 0: no gate
 };
 
 struct ekfslam_ctx {
@@ -122,6 +136,7 @@ struct ekfslam_ctx {
     // the context's own frame buffers while caller-owned ones are bound (ekfslam_bind_frame)
     double* own_zc; uint8_t* own_mflags; double* own_u; int own_n_u;
     DevEval ev;
+    DevCamUpd cu;
 };
 
 // W is stored panel-major: element (row t, column c) of a filter lives at ((c / 64) * wrows + t) * EKF_WPAD + c % 64.
@@ -193,3 +208,5 @@ void launch_world_uniforms(ekfslam_ctx* c, int t);
 void launch_mm_plan(ekfslam_ctx* c, int min_features);
 // mode 0: score filters [b0, b0+nb) against frame t of the world; mode 1: map export of filters [b0, b0+nb)
 void launch_eval(ekfslam_ctx* c, int mode, int t, int b0, int nb);
+// camera-state update of (x_k_k, P) (which 0) or (x_k_km1, P) (which 1) from the staged c->cu, then the downdate
+void launch_cam_update(ekfslam_ctx* c, int which);

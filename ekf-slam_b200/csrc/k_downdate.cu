@@ -623,9 +623,9 @@ void launch_downdate(ekfslam_ctx* c, int slot) {
     const int nt = (v.nmax + TM - 1) / TM;
     const int T = nt * (nt + 1) / 2;
     KScope ks(c, slot);
-    // ring depth / P buffers by update kind: the hi update usually stacks few rows (short K loops, the kernel
-    // streams P), the li update many.
-    const bool cfgB = slot == KT_DOWNDATE_HI;
+    // ring depth / P buffers by update kind: the hi update and the camera-state update stack few rows (short K loops,
+    // the kernel streams P), the li update many.
+    const bool cfgB = slot != KT_DOWNDATE;
     const int S = cfgB ? 2 : 4, NX = cfgB ? 2 : 1;
     // filters are processed in groups small enough for the per-CTA tile metadata (8 B per tile) to stay
     // within the shared-memory budget of two CTAs per SM

@@ -349,6 +349,31 @@ int ekfslam_reset_eval(ekfslam_ctx* ctx);
  * packed (xx, yx, yy, zx, zy, zz); NaN for empty and not evaluable slots.  Either pointer may be NULL. */
 int ekfslam_map_cartesian(ekfslam_ctx* ctx, int b0, int nb, double* p, double* cov);
 
+/* ---- camera-state measurement update (EXTENSION: the reference has no such update) ---- */
+/* A metric sensor on the camera state: a position fix, a velocity, an angular rate, or any linear combination of
+ * x[0:13] = [r q v w].  For filter b with on[b] != 0, m rows (1 <= m <= min(13, 2 N_max)):
+ *   z_b = H_b x[0:13] + v,  v ~ N(0, R_b),  H_b: m x 13,  R_b: m x m SPD (its lower triangle is read).
+ * The update is mc/update.m:3-32 with the full Jacobian [H_b | 0], computed the way the feature updates compute it:
+ *   nu = z - H x,  S = H P H' + R = L L',  W = inv(L) (H P),  y = inv(L) nu,  x+ = x + W' y,
+ *   then q+ <- q+/|q+| and P+ = J P J' - (W J')' (W J') with J = blkdiag(I3, normJac(q+), I)  (mc/update.m:18-24);
+ *   NIS = nu' inv(S) nu = |y|^2.
+ * which: 0 updates (x_k_k, P) (after ekfslam_step or ekfslam_update_hi); 1 updates (x_k_km1, P) (between
+ * ekfslam_predict and ekfslam_measure, so that matching, RANSAC and the li update all see the aided prior).  P is one
+ * buffer; the other x buffer is not touched.
+ * Per filter a status is recorded (EKFSLAM_CAM_*): 0 applied, 1 not selected (on[b] == 0 or b outside [b0, b0+nb)),
+ * 2 gated out (gate > 0 and NIS > gate), 3 S not SPD (a Cholesky pivot not > 0) or NIS not finite.  Statuses 1-3 leave
+ * every byte of that filter's state unchanged.  NIS is recorded for statuses 0 and 2 and is NaN otherwise.
+ * A nonlinear sensor h(x) is passed linearised: H = dh/dx at the estimate x^ and z_eff = z - h(x^) + H x^.
+ * The cost is one pass of the covariance downdate over P (one read and one write of P).  Stream-ordered, no
+ * synchronisation; its staging buffers are allocated on the first call. */
+enum { EKFSLAM_CAM_APPLIED = 0, EKFSLAM_CAM_OFF = 1, EKFSLAM_CAM_GATED = 2, EKFSLAM_CAM_NOT_SPD = 3 };
+/* H [nb][m][13] row-major, z [nb][m], R [nb][m][m], on [nb] (NULL = all); gate <= 0: no gate.
+ * ERR_INVALID: m outside [1, min(13, 2 N_max)], which not 0 or 1, a bad [b0, b0+nb), a NULL H, z or R. */
+int ekfslam_update_camera(ekfslam_ctx* ctx, int b0, int nb, int m, const double* H, const double* z,
+                          const double* R, const uint8_t* on, double gate, int which);
+/* last call's per-filter NIS [nb] and status [nb] (either may be NULL); ERR_STATE before the first call */
+int ekfslam_download_camera_update(ekfslam_ctx* ctx, int b0, int nb, double* nis, int32_t* status);
+
 /* ---- measurement hooks ------------------------------------------------------ */
 /* bracket every kernel launch with a CUDA event pair on the context's stream and accumulate the
  * elapsed time per kernel; enabling again resets the accumulators, on=0 removes the events */
