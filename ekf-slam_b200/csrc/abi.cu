@@ -852,18 +852,22 @@ int ekfslam_step_host(ekfslam_ctx* c, int match_mode, const double* zc, const ui
     return EKFSLAM_OK;
 }
 
+static int ensure_scratch(ekfslam_ctx* c, size_t need) {
+    if (need > c->pin_bytes) {
+        if (c->pin) { CK(cudaStreamSynchronize(c->stream)); CK(cudaFree(c->pin)); c->pin = nullptr; c->pin_bytes = 0; }
+        CK(cudaMalloc(&c->pin, need));
+        c->pin_bytes = need;
+    }
+    return EKFSLAM_OK;
+}
+
 int ekfslam_reset_filters(ekfslam_ctx* c, int b0, int nb, const double* xv, const double* Pxv) {
     NEED_CTX(c);
     if (c->own_zc) return fail(EKFSLAM_ERR_STATE, "frame buffers are bound to caller memory (ekfslam_unbind_frame first)");
     if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
     if (!xv || !Pxv) return fail(EKFSLAM_ERR_INVALID, "xv / Pxv is null");
     DevView& v = c->v;
-    const size_t need = sizeof(double) * (13 + 169);
-    if (need > c->pin_bytes) {
-        if (c->pin) { CK(cudaStreamSynchronize(c->stream)); CK(cudaFree(c->pin)); c->pin = nullptr; c->pin_bytes = 0; }
-        CK(cudaMalloc(&c->pin, need));
-        c->pin_bytes = need;
-    }
+    if (int r = ensure_scratch(c, sizeof(double) * (13 + 169))) return r;
     double* d = (double*)c->pin;
     CK(cudaMemcpyAsync(d, xv, sizeof(double) * 13, cudaMemcpyHostToDevice, c->stream));
     CK(cudaMemcpyAsync(d + 13, Pxv, sizeof(double) * 169, cudaMemcpyHostToDevice, c->stream));
@@ -891,12 +895,7 @@ int ekfslam_add_features(ekfslam_ctx* c, int b0, int nb, const double* uvd, cons
     if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
     if (!uvd) return fail(EKFSLAM_ERR_INVALID, "uvd is null");
     // staging buffers for the pixels / mask (grown on demand, freed with the context)
-    const size_t need = sizeof(double) * 2 * (size_t)nb + (size_t)nb;
-    if (need > c->pin_bytes) {
-        if (c->pin) { CK(cudaStreamSynchronize(c->stream)); CK(cudaFree(c->pin)); c->pin = nullptr; c->pin_bytes = 0; }
-        CK(cudaMalloc(&c->pin, need));
-        c->pin_bytes = need;
-    }
+    if (int r = ensure_scratch(c, sizeof(double) * 2 * (size_t)nb + (size_t)nb)) return r;
     double* d_uvd = (double*)c->pin;
     uint8_t* d_add = (uint8_t*)(d_uvd + 2 * (size_t)nb);
     CK(cudaMemcpyAsync(d_uvd, uvd, sizeof(double) * 2 * nb, cudaMemcpyHostToDevice, c->stream));
@@ -904,15 +903,6 @@ int ekfslam_add_features(ekfslam_ctx* c, int b0, int nb, const double* uvd, cons
     launch_add_features(c, b0, nb, d_uvd, 2, add ? d_add : nullptr, nullptr, 0, nullptr, 0, std_pxl, initial_rho, std_rho);
     LAUNCHED();
     CK(cudaStreamSynchronize(c->stream));
-    return EKFSLAM_OK;
-}
-
-static int ensure_scratch(ekfslam_ctx* c, size_t need) {
-    if (need > c->pin_bytes) {
-        if (c->pin) { CK(cudaStreamSynchronize(c->stream)); CK(cudaFree(c->pin)); c->pin = nullptr; c->pin_bytes = 0; }
-        CK(cudaMalloc(&c->pin, need));
-        c->pin_bytes = need;
-    }
     return EKFSLAM_OK;
 }
 

@@ -147,6 +147,14 @@ __host__ __device__ __forceinline__ size_t w_at(int wrows, int t, int c) {
     return ((size_t)(c >> 6) * wrows + t) * EKF_WPAD + (c & 63);
 }
 
+// Columns 3..6 of one row of W <- . Jt' (w = the row's column 3, Jt row-major 4x4): the update's normalisation Jacobian
+// J = blkdiag(I3, Jt, I) folded into W, since P+ = J (P - W'W) J' = J P J' - (W J')' (W J')  (mc/update.m:20-22).
+__device__ __forceinline__ void w_fold_jt(double* w, const double* Jt) {
+    const double w3 = w[0], w4 = w[1], w5 = w[2], w6 = w[3];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) w[i] = w3 * Jt[i * 4 + 0] + w4 * Jt[i * 4 + 1] + w5 * Jt[i * 4 + 2] + w6 * Jt[i * 4 + 3];
+}
+
 #define EKF_TRI(nic, s) (((nic) * ((nic) + 1)) / 2 + (s))
 
 // The update's Cholesky runs lock-step over all filters (one launch per phase, k_chol_big.cu) for few filters with a

@@ -16,7 +16,7 @@
 //   2. a thread per state column c < ld: g = H P[0:13, c] from the coalesced rows 0..12 (P is exactly symmetric in
 //      memory), W[:, c] = inv(L) g (padding columns [n, ld) written as zero), x[c] += sum_a W[a][c] y[a].
 //   3. normJac(q+) from the un-normalised quaternion, q+ <- q+/|q+| (mc/update.m:18,24), rows a < m of W get columns
-//      3..6 <- . Jt' (the arithmetic of k_wfix), jn[b] = Jt, ktot[b] = m.
+//      3..6 <- . Jt' (w_fold_jt, as in k_wfix), jn[b] = Jt, ktot[b] = m.
 // A filter whose status is not 0 ends with ktot[b] = 0 (the downdate skips it) and is not written.
 __global__ void __launch_bounds__(CU_THREADS) k_cam_update(DevView v, DevCamUpd cu, int which) {
     const int b = blockIdx.x;
@@ -152,25 +152,9 @@ __global__ void __launch_bounds__(CU_THREADS) k_cam_update(DevView v, DevCamUpd 
         if (incol) x[c] += xa;
     }
     __syncthreads();
-    if (tid == 0) {
-        // normJac(q+) (mc/normJac.m) from the un-normalised quaternion, then q+ <- q+/|q+|  (mc/update.m:18,24)
-        const double r = x[3], qx = x[4], qy = x[5], qz = x[6];
-        const double nn = r * r + qx * qx + qy * qy + qz * qz;
-        const double sc = 1.0 / (nn * sqrt(nn));  // (.)^(-3/2)
-        Jt[0] = sc * (qx * qx + qy * qy + qz * qz); Jt[1] = sc * (-r * qx); Jt[2] = sc * (-r * qy); Jt[3] = sc * (-r * qz);
-        Jt[4] = sc * (-qx * r); Jt[5] = sc * (r * r + qy * qy + qz * qz); Jt[6] = sc * (-qx * qy); Jt[7] = sc * (-qx * qz);
-        Jt[8] = sc * (-qy * r); Jt[9] = sc * (-qy * qx); Jt[10] = sc * (r * r + qx * qx + qz * qz); Jt[11] = sc * (-qy * qz);
-        Jt[12] = sc * (-qz * r); Jt[13] = sc * (-qz * qx); Jt[14] = sc * (-qz * qy); Jt[15] = sc * (r * r + qx * qx + qy * qy);
-        const double nrm = sqrt(nn);
-        x[3] = r / nrm; x[4] = qx / nrm; x[5] = qy / nrm; x[6] = qz / nrm;
-    }
+    if (tid == 0) normjac_normalize(x, Jt);
     __syncthreads();
-    if (tid < m) {   // W <- W J' on columns 3..6 (k_wfix)
-        double* w = W + w_at(v.wrows, tid, 3);
-        const double w3 = w[0], w4 = w[1], w5 = w[2], w6 = w[3];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) w[i] = w3 * Jt[i * 4 + 0] + w4 * Jt[i * 4 + 1] + w5 * Jt[i * 4 + 2] + w6 * Jt[i * 4 + 3];
-    }
+    if (tid < m) w_fold_jt(W + w_at(v.wrows, tid, 3), Jt);
     if (tid < 16) v.jn[(size_t)b * 16 + tid] = Jt[tid];
     if (tid == 0) v.ktot[b] = m;
 }

@@ -101,55 +101,6 @@ __device__ __forceinline__ void cb_store(double* __restrict__ dst, int kmax, int
 }
 
 // ---------------------------------------------------------------------------------------
-// 16x16 Cholesky + inverse by ONE warp, the block held in registers (lane i = row i, lanes 16..31 mirror 0..15), pivots
-// exchanged with shuffles, rsqrt pivots - the scheme of the smaller Cholesky kernels.  Blk: shared, lower triangle in /
-// L out; Di [16][17]: inv(L), zeros above the diagonal.
-// ---------------------------------------------------------------------------------------
-__device__ __forceinline__ bool chol16_warp(double* __restrict__ Blk, int pitch, double* __restrict__ Di) {
-    const unsigned full = 0xffffffffu;
-    const int lane = threadIdx.x & 31, i = lane & 15;
-    double a[16], rd[16];
-#pragma unroll
-    for (int c = 0; c < 16; ++c) a[c] = (c <= i) ? Blk[i * pitch + c] : 0.0;
-    bool bad = false;
-#pragma unroll
-    for (int c = 0; c < 16; ++c) {
-        const double piv = __shfl_sync(full, a[c], c);
-        bad = bad || !(piv > 0.0);
-        const double rs = rsqrt(piv);
-        rd[c] = rs;
-        const double lic = (i == c) ? piv * rs : a[c] * rs;
-        a[c] = lic;
-#pragma unroll
-        for (int j = c + 1; j < 16; ++j) {
-            const double ljc = __shfl_sync(full, lic, j);
-            a[j] -= lic * ljc;
-        }
-    }
-    if (lane < 16) {
-#pragma unroll
-        for (int c = 0; c < 16; ++c)
-            if (c <= i) Blk[i * pitch + c] = a[c];
-    }
-    __syncwarp();
-    // column c = lane of inv(L) by forward substitution
-    const int c = i;
-    double x[16];
-#pragma unroll
-    for (int ii = 0; ii < 16; ++ii) {
-        double sacc = 0.0;
-#pragma unroll
-        for (int t = 0; t < ii; ++t) sacc += Blk[ii * pitch + t] * x[t];
-        x[ii] = (ii == c) ? rd[ii] : ((ii > c) ? -sacc * rd[ii] : 0.0);
-    }
-    if (lane < 16) {
-#pragma unroll
-        for (int ii = 0; ii < 16; ++ii) Di[ii * 17 + c] = x[ii];
-    }
-    return bad;
-}
-
-// ---------------------------------------------------------------------------------------
 // panel j0: diagonal block factor + inverse (every CTA), panel block product (CTAs 1..)
 // grid = (1 + blocks below the panel, B), 256 threads, dynamic shared memory 3 blocks
 // The 64x64 diagonal block is factored in shared memory in four 16-wide steps (warp 0 factors and inverts the 16x16

@@ -16,6 +16,14 @@
 
 #define NB 16
 
+// index e of a lower triangle stored by rows -> (r, c), c <= r
+__device__ __forceinline__ void tri_unrank(int e, int& r, int& c) {
+    r = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
+    while ((r + 1) * (r + 2) / 2 <= e) ++r;
+    while (r * (r + 1) / 2 > e) --r;
+    c = e - r * (r + 1) / 2;
+}
+
 // S = G_sel H_sel' + I, lower triangle at feature-pair granularity: pair e -> (fa >= fb) -> one 2x2 block.
 // STAGED: the per-feature operands of the pair loop (feature index, state offset, block width, compact Jacobian) come from
 // shared memory (k_upd_S stages them once per filter), so the only global loads left per pair are the 2 x 13 entries of G,
@@ -31,11 +39,8 @@ __device__ __forceinline__ void upd_S_pairs(const DevView& v, int b, int ns, int
     double* __restrict__ S = v.Sb + (size_t)b * kmax * kmax;
     const int npair = ns * (ns + 1) / 2;
     for (int e = first; e < npair; e += stride) {
-        // unrank e -> (fa, fb), fa >= fb
-        int fa = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
-        while ((fa + 1) * (fa + 2) / 2 <= e) ++fa;
-        while (fa * (fa + 1) / 2 > e) --fa;
-        const int fb = e - fa * (fa + 1) / 2;
+        int fa, fb;   // fa >= fb
+        tri_unrank(e, fa, fb);
         int ia, off, w;
         const double* __restrict__ H;
         if (STAGED) {
@@ -193,52 +198,7 @@ __global__ void __launch_bounds__(128) k_chol(DevView v, int kskip) {
         }
         __syncthreads();
         if (warp == 0) {
-            // Cholesky of the NB x NB diagonal block in registers: lane i holds row i (lanes 16-31 mirror
-            // lanes 0-15 so that every shuffle is full-warp); column c is broadcast by shuffles.
-            const unsigned full_mask = 0xffffffffu;
-            const int i = lane & (NB - 1);
-            double a[NB];
-#pragma unroll
-            for (int c = 0; c < NB; ++c) a[c] = D[i * (NB + 1) + c];
-            bool bad = false;
-            double rdiag[NB];  // 1 / L[c][c]: one rsqrt per pivot replaces the sqrt and every division
-#pragma unroll
-            for (int c = 0; c < NB; ++c) {
-                const double piv = __shfl_sync(full_mask, a[c], c);
-                bad = bad || !(piv > 0.0);
-                const double rs = rsqrt(piv);
-                rdiag[c] = rs;
-                const double lic = (i == c) ? piv * rs : a[c] * rs;  // rows above the diagonal carry don't-care values
-                a[c] = lic;
-#pragma unroll
-                for (int j = c + 1; j < NB; ++j) {
-                    const double ljc = __shfl_sync(full_mask, lic, j);
-                    a[j] -= lic * ljc;
-                }
-            }
-            if (bad && lane == 0) s_bad = 1;
-            if (lane < NB) {
-#pragma unroll
-                for (int c = 0; c < NB; ++c) D[i * (NB + 1) + c] = (c <= i) ? a[c] : 0.0;
-            }
-            __syncwarp();
-            // inverse of the triangular block: lane c solves column c by forward substitution; every lane
-            // reads the same L entry at the same time (shared-memory broadcast)
-            {
-                const int c = i;
-                double x[NB];
-#pragma unroll
-                for (int ii = 0; ii < NB; ++ii) {
-                    double sacc = 0.0;
-#pragma unroll
-                    for (int t = 0; t < ii; ++t) sacc += D[ii * (NB + 1) + t] * x[t];
-                    x[ii] = (ii == c) ? rdiag[ii] : ((ii > c) ? -sacc * rdiag[ii] : 0.0);
-                }
-                if (lane < NB) {
-#pragma unroll
-                    for (int ii = 0; ii < NB; ++ii) Di[ii * (NB + 1) + c] = x[ii];
-                }
-            }
+            if (chol16_warp(D, NB + 1, Di) && lane == 0) s_bad = 1;
         }
         __syncthreads();
         for (int e = tid; e < nb * nb; e += blockDim.x) {
@@ -272,10 +232,8 @@ __global__ void __launch_bounds__(128) k_chol(DevView v, int kskip) {
             const int mt = (m + 3) / 4;  // 4x4 micro tiles
             const int ntile = mt * (mt + 1) / 2;
             for (int e = tid; e < ntile; e += blockDim.x) {
-                int ti = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
-                while ((ti + 1) * (ti + 2) / 2 <= e) ++ti;
-                while (ti * (ti + 1) / 2 > e) --ti;
-                const int tj = e - ti * (ti + 1) / 2;
+                int ti, tj;
+                tri_unrank(e, ti, tj);
                 double acc[4][4];
 #pragma unroll
                 for (int a = 0; a < 4; ++a)
@@ -472,20 +430,6 @@ __device__ __forceinline__ void chs_inv_store(double* Ls, int I0, int nb, int pa
     }
 }
 
-#ifdef CHS_PROF
-// debug build only (-DCHS_PROF): cycles of thread 0 between the barriers of each phase, summed over the CTAs of the
-// 112-row variant; read back with ekfslam_debug_chs_prof
-__device__ unsigned long long g_chs_prof[16];
-extern "C" int ekfslam_debug_chs_prof(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    if (out) cudaMemcpyFromSymbol(out, g_chs_prof, sizeof(g_chs_prof));
-    if (reset) { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(g_chs_prof, z, sizeof(z)); }
-    return 0;
-}
-#define CHS_MARK(ph) do { if (KM == CHS_KM && KMIN == 0 && tid == 0) { const unsigned t1_ = (unsigned)clock(); atomicAdd(&g_chs_prof[ph], (unsigned long long)(t1_ - t0_)); t0_ = t1_; } } while (0)
-#else
-#define CHS_MARK(ph) do { } while (0)
-#endif
 template <int KM, int CHS_T, int KMIN, int MINB = 1>
 __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
     extern __shared__ __align__(16) double sm[];
@@ -503,10 +447,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
     double* Pn = DiA + 2 * NB * (NB + 1);              // [NB][KM] transposed panel of the trailing update / vectors
     __shared__ int s_bad;
     if (tid == 0) s_bad = 0;
-#ifdef CHS_PROF
-    unsigned t0_ = (unsigned)clock();
-    if (KM == CHS_KM && KMIN == 0 && tid == 0) atomicAdd(&g_chs_prof[15], 1ull);
-#endif
     // every element of the lower triangle is its own 8-byte asynchronous copy (LDGSTS.64): ~20 independent copies in
     // flight per thread instead of a dependent DRAM round trip per row (ncu: 11 % of the kernel's samples sat on the
     // plain load loop; k_chol 1.42 -> 1.33 ms)
@@ -515,7 +455,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
     cp_async_commit();
     cp_async_wait<0>();
     __syncthreads();
-    CHS_MARK(0);
 
     for (int j0 = 0; j0 < k; j0 += NB) {
         const int nb = min(NB, k - j0);
@@ -532,57 +471,12 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
             Di[r * (NB + 1) + c] = 0.0;
         }
         __syncthreads();
-        CHS_MARK(1);
         if (warp == 0) {
-            // as in k_chol: lane i holds row i of the block, pivots by rsqrt, then the triangular inverse
-            const unsigned full_mask = 0xffffffffu;
-            const int i = lane & (NB - 1);
-            double a[NB];
-#pragma unroll
-            for (int c = 0; c < NB; ++c) a[c] = D[i * (NB + 1) + c];
-            bool bad = false;
-            double rdiag[NB];
-#pragma unroll
-            for (int c = 0; c < NB; ++c) {
-                const double piv = __shfl_sync(full_mask, a[c], c);
-                bad = bad || !(piv > 0.0);
-                const double rs = rsqrt(piv);
-                rdiag[c] = rs;
-                const double lic = (i == c) ? piv * rs : a[c] * rs;
-                a[c] = lic;
-#pragma unroll
-                for (int j = c + 1; j < NB; ++j) {
-                    const double ljc = __shfl_sync(full_mask, lic, j);
-                    a[j] -= lic * ljc;
-                }
-            }
-            if (bad && lane == 0) s_bad = 1;
-            CHS_MARK(8);
-            if (lane < NB) {
-#pragma unroll
-                for (int c = 0; c < NB; ++c) D[i * (NB + 1) + c] = (c <= i) ? a[c] : 0.0;
-            }
-            __syncwarp();
-            {
-                const int c = i;
-                double x[NB];
-#pragma unroll
-                for (int ii = 0; ii < NB; ++ii) {
-                    double sacc = 0.0;
-#pragma unroll
-                    for (int t = 0; t < ii; ++t) sacc += D[ii * (NB + 1) + t] * x[t];
-                    x[ii] = (ii == c) ? rdiag[ii] : ((ii > c) ? -sacc * rdiag[ii] : 0.0);
-                }
-                if (lane < NB) {
-#pragma unroll
-                    for (int ii = 0; ii < NB; ++ii) Di[ii * (NB + 1) + c] = x[ii];
-                }
-            }
+            if (chol16_warp(D, NB + 1, Di) && lane == 0) s_bad = 1;
         }
         else if (inv_prev) chs_inv_compute(Ls, Dip, j0 - NB, NB, warp - 1, lane, res);
         __syncthreads();
         if (inv_prev) chs_inv_store(Ls, j0 - NB, NB, warp - 1, lane, res);
-        CHS_MARK(2);
         // the diagonal block of X replaces the one of L (the panel solve and the inverse phase only use Di)
         for (int e = tid; e < nb * nb; e += CHS_T) {
             const int r = e / nb, c = e - r * nb;
@@ -614,7 +508,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
             for (int c = 0; c < NB; ++c) PT[c * KM + m + tid] = 0.0;
         }
         __syncthreads();
-        CHS_MARK(3);
         // trailing update of the lower triangle: S[i][c] -= sum_t L[i][j0+t] L[c][j0+t]   (4x4 micro tiles)
         if (m > 0) {
             const int mt = (m + 3) / 4;
@@ -665,7 +558,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
             }
         }
         __syncthreads();
-        CHS_MARK(4);
     }
 
     // the last block row of inv(L) (the others were formed under the pivot chains above): all warps, one pair each
@@ -678,7 +570,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
         __syncthreads();
         if (act) chs_inv_store(Ls, I0, k - I0, warp, lane, res);
         __syncthreads();
-        CHS_MARK(6);
     }
     // inv(L) to global memory with explicit zeros above the diagonal (k_gemm streams it unmasked)
     for (int r = warp; r < k; r += nwarps)
@@ -713,7 +604,6 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
         for (; a < k; ++a) s0 += Ls[tri(a, t)] * ys[a];
         cv[t] = (s0 + s1) + (s2 + s3);
     }
-    CHS_MARK(7);
     if (tid == 0 && s_bad) atomicOr(&v.stats[b].status, 2);
 }
 
@@ -1113,21 +1003,9 @@ __global__ void __launch_bounds__(256, 3) k_gemm(DevView v, int finalize, int ks
             __syncthreads();
             if (tid < TM && c0 + tid < n) x[c0 + tid] += (xred[tid] + xred[tid + 64]) + (xred[tid + 128] + xred[tid + 192]);
             if (c0 == 0 && finalize) {
-                // this block owns state entries 0..63: normJac(q+) (mc/normJac.m) from the un-normalised
-                // quaternion, then q+ <- q+/|q+|  (mc/update.m:18,24)
+                // this block owns state entries 0..63, the quaternion among them
                 __syncthreads();
-                if (tid == 0) {
-                    const double r = x[3], qx = x[4], qy = x[5], qz = x[6];
-                    const double nn = r * r + qx * qx + qy * qy + qz * qz;
-                    const double sc = 1.0 / (nn * sqrt(nn));  // (.)^(-3/2)
-                    double* J = v.jnt + (size_t)b * 16;
-                    J[0] = sc * (qx * qx + qy * qy + qz * qz); J[1] = sc * (-r * qx); J[2] = sc * (-r * qy); J[3] = sc * (-r * qz);
-                    J[4] = sc * (-qx * r); J[5] = sc * (r * r + qy * qy + qz * qz); J[6] = sc * (-qx * qy); J[7] = sc * (-qx * qz);
-                    J[8] = sc * (-qy * r); J[9] = sc * (-qy * qx); J[10] = sc * (r * r + qx * qx + qz * qz); J[11] = sc * (-qy * qz);
-                    J[12] = sc * (-qz * r); J[13] = sc * (-qz * qx); J[14] = sc * (-qz * qy); J[15] = sc * (r * r + qx * qx + qy * qy);
-                    const double nrm = sqrt(nn);
-                    x[3] = r / nrm; x[4] = qx / nrm; x[5] = qy / nrm; x[6] = qz / nrm;
-                }
+                if (tid == 0) normjac_normalize(x, v.jnt + (size_t)b * 16);
             }
         }
         it = 0; ++cb;
@@ -1207,19 +1085,7 @@ __global__ void __launch_bounds__(128, MINB) k_w_small(DevView v, int finalize) 
     }
     if (finalize) {
         __syncthreads();
-        if (tid == 0) {
-            // normJac(q+) (mc/normJac.m) from the un-normalised quaternion, then q+ <- q+/|q+|  (mc/update.m:18,24)
-            const double r = x[3], qx = x[4], qy = x[5], qz = x[6];
-            const double nn = r * r + qx * qx + qy * qy + qz * qz;
-            const double sc = 1.0 / (nn * sqrt(nn));  // (.)^(-3/2)
-            double* J = v.jnt + (size_t)b * 16;
-            J[0] = sc * (qx * qx + qy * qy + qz * qz); J[1] = sc * (-r * qx); J[2] = sc * (-r * qy); J[3] = sc * (-r * qz);
-            J[4] = sc * (-qx * r); J[5] = sc * (r * r + qy * qy + qz * qz); J[6] = sc * (-qx * qy); J[7] = sc * (-qx * qz);
-            J[8] = sc * (-qy * r); J[9] = sc * (-qy * qx); J[10] = sc * (r * r + qx * qx + qz * qz); J[11] = sc * (-qy * qz);
-            J[12] = sc * (-qz * r); J[13] = sc * (-qz * qx); J[14] = sc * (-qz * qy); J[15] = sc * (r * r + qx * qx + qy * qy);
-            const double nrm = sqrt(nn);
-            x[3] = r / nrm; x[4] = qx / nrm; x[5] = qy / nrm; x[6] = qz / nrm;
-        }
+        if (tid == 0) normjac_normalize(x, v.jnt + (size_t)b * 16);
     }
 }
 
@@ -1236,12 +1102,7 @@ __global__ void __launch_bounds__(128) k_wfix(DevView v) {
     __shared__ double Jt[16];
     if (threadIdx.x < 16) Jt[threadIdx.x] = v.jnt[(size_t)b * 16 + threadIdx.x];
     __syncthreads();
-    for (int a = threadIdx.x; a < k; a += blockDim.x) {
-        double* w = W + w_at(v.wrows, a, 3);
-        const double w3 = w[0], w4 = w[1], w5 = w[2], w6 = w[3];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) w[i] = w3 * Jt[i * 4 + 0] + w4 * Jt[i * 4 + 1] + w5 * Jt[i * 4 + 2] + w6 * Jt[i * 4 + 3];
-    }
+    for (int a = threadIdx.x; a < k; a += blockDim.x) w_fold_jt(W + w_at(v.wrows, a, 3), Jt);
     if (threadIdx.x < 16 && k > 0) v.jn[(size_t)b * 16 + threadIdx.x] = Jt[threadIdx.x];
     if (threadIdx.x == 0) v.ktot[b] = k;
 }

@@ -14,6 +14,20 @@ EKF_DEV void q2r_dev(const double* q, double* R) {
     R[6] = 2.0 * (z * x - r * y);         R[7] = 2.0 * (y * z + r * x);         R[8] = r * r - x * x - y * y + z * z;
 }
 
+// mc/normJac.m + mc/update.m:18,24 — J[16] (row-major 4x4) = normJac(q+) of the un-normalised quaternion q+ = x[3..6],
+// then q+ <- q+/|q+|.  Thread-0 code of the update epilogues.
+EKF_DEV void normjac_normalize(double* x, double* J) {
+    const double r = x[3], qx = x[4], qy = x[5], qz = x[6];
+    const double nn = r * r + qx * qx + qy * qy + qz * qz;
+    const double sc = 1.0 / (nn * sqrt(nn));  // (.)^(-3/2)
+    J[0] = sc * (qx * qx + qy * qy + qz * qz); J[1] = sc * (-r * qx); J[2] = sc * (-r * qy); J[3] = sc * (-r * qz);
+    J[4] = sc * (-qx * r); J[5] = sc * (r * r + qy * qy + qz * qz); J[6] = sc * (-qx * qy); J[7] = sc * (-qx * qz);
+    J[8] = sc * (-qy * r); J[9] = sc * (-qy * qx); J[10] = sc * (r * r + qx * qx + qz * qz); J[11] = sc * (-qy * qz);
+    J[12] = sc * (-qz * r); J[13] = sc * (-qz * qx); J[14] = sc * (-qz * qy); J[15] = sc * (r * r + qx * qx + qy * qy);
+    const double nrm = sqrt(nn);
+    x[3] = r / nrm; x[4] = qx / nrm; x[5] = qy / nrm; x[6] = qz / nrm;
+}
+
 // mc/distort_fm.m:22-38 — undistorted pixel -> distorted pixel (10 Newton steps on
 // rd + k1 rd^3 + k2 rd^5 = ru).  The loop leaves early once rd reaches a fixed point:
 // from there every further step of the reference reproduces the same rd bit for bit.

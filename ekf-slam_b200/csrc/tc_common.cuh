@@ -1,5 +1,6 @@
 // Shared building blocks of the tensor-core kernels (k_w, k_downdate*): DMMA wrapper, cp.async ring
-// helpers, mbarrier / bulk-copy wrappers, lower-triangle tile decoding.
+// helpers, mbarrier / bulk-copy wrappers, lower-triangle tile decoding; and the 16-wide warp Cholesky of the
+// update's diagonal blocks.
 #pragma once
 #include "common.cuh"
 
@@ -30,6 +31,56 @@ __device__ __forceinline__ void cp_async8(double* smem_dst, const double* gmem_s
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// ---------------------------------------------------------------------------------------
+// 16x16 Cholesky + inverse by ONE warp (the diagonal blocks of k_chol, k_chol_sm and k_cb_diagpanel), the block held in
+// registers (lane i = row i, lanes 16..31 mirror 0..15 so that every shuffle is full-warp), column c broadcast by
+// shuffles, one rsqrt per pivot in place of the sqrt and every division.  Blk: shared, the lower triangle in (the upper
+// one is not read), L out with zeros above the diagonal; rows past the data must be padded with the identity.
+// Di [16][17]: inv(L), all 16 x 16 entries written (zeros above the diagonal).  Returns true for a pivot that is not > 0.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ bool chol16_warp(double* __restrict__ Blk, int pitch, double* __restrict__ Di) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31, i = lane & 15;
+    double a[16], rd[16];
+#pragma unroll
+    for (int c = 0; c < 16; ++c) a[c] = (c <= i) ? Blk[i * pitch + c] : 0.0;
+    bool bad = false;
+#pragma unroll
+    for (int c = 0; c < 16; ++c) {
+        const double piv = __shfl_sync(full, a[c], c);
+        bad = bad || !(piv > 0.0);
+        const double rs = rsqrt(piv);
+        rd[c] = rs;
+        const double lic = (i == c) ? piv * rs : a[c] * rs;  // rows above the diagonal carry don't-care values
+        a[c] = lic;
+#pragma unroll
+        for (int j = c + 1; j < 16; ++j) {
+            const double ljc = __shfl_sync(full, lic, j);
+            a[j] -= lic * ljc;
+        }
+    }
+    if (lane < 16) {
+#pragma unroll
+        for (int c = 0; c < 16; ++c) Blk[i * pitch + c] = (c <= i) ? a[c] : 0.0;
+    }
+    __syncwarp();
+    // column c = lane of inv(L) by forward substitution; every lane reads the same L entry at the same time (broadcast)
+    const int c = i;
+    double x[16];
+#pragma unroll
+    for (int ii = 0; ii < 16; ++ii) {
+        double sacc = 0.0;
+#pragma unroll
+        for (int t = 0; t < ii; ++t) sacc += Blk[ii * pitch + t] * x[t];
+        x[ii] = (ii == c) ? rd[ii] : ((ii > c) ? -sacc * rd[ii] : 0.0);
+    }
+    if (lane < 16) {
+#pragma unroll
+        for (int ii = 0; ii < 16; ++ii) Di[ii * 17 + c] = x[ii];
+    }
+    return bad;
+}
 
 
 struct DTile {
