@@ -251,10 +251,8 @@ __global__ void __launch_bounds__(256) k_cb_trail(DevView v, int j0) {
     const int i1 = j0 + CB;
     if (i1 >= k) return;
     const int e = blockIdx.x;
-    int ta = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-    while ((ta + 1) * (ta + 2) / 2 <= e) ++ta;
-    while (ta * (ta + 1) / 2 > e) --ta;
-    const int tb = e - ta * (ta + 1) / 2;
+    int ta, tb;
+    tri_unrank(e, ta, tb);
     const int r0 = i1 + ta * CB, c0 = i1 + tb * CB;
     if (r0 >= k) return;
     const int kmax = v.kmax;

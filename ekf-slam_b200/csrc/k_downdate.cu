@@ -5,22 +5,18 @@
 // tile itself: columns 3..6 of tile column 0 and rows 3..6 of tile (0,0).  0.5P + 0.5P' (:14) is the identity
 // because the lower triangle is authoritative and every tile is stored together with its mirror image.
 //
-// Two kernels, same arithmetic and summation order (k ascending, DMMA m8n8k4):
-//   k_downdate_ws2  (default) persistent, warp-specialised, 2 CTAs per SM: a producer warp streams the W panels with
-//                   bulk asynchronous copies (cp.async.bulk -> SASS UBLKCP, one per panel and stage thanks to the
-//                   panel-major W layout) on a 4-stage mbarrier ring that keeps running across tile boundaries; 8
-//                   consumer warps issue the DMMAs; 4 epilogue warps prefetch the next P tile into shared memory and
-//                   store the finished tile and its mirror image while the consumers are already in the next K loop.
-//   k_downdate_tile (the fallback for shapes whose tile list does not fit the persistent kernel's shared memory:
-//                   n_max > 4352 for the li update, n_max > 4608 for the hi update) one CTA per tile, cp.async (LDGSTS) ring.
+// One kernel, k_downdate_ws2: persistent, warp-specialised, 2 CTAs per SM, for every update and shape.  A producer warp
+// streams the W panels with bulk asynchronous copies (cp.async.bulk -> SASS UBLKCP, one per panel and stage thanks to
+// the panel-major W layout) on an mbarrier ring that keeps running across tile boundaries; 8 consumer warps issue the
+// DMMAs (m8n8k4, k ascending); 4 epilogue warps prefetch the next P tile into shared memory and store the finished tile
+// and its mirror image while the consumers are already in the next K loop.
 #include <cstdlib>
 #include "model.cuh"
 #include "tc_common.cuh"
 
 #define WS_CONSUMERS 8
-#define XP_ 66   // row pitch (doubles) of the shared P tile buffer X of k_downdate_ws2 (= XP below)
+#define XP 66   // row pitch (doubles) of the shared P tile buffer X: rows stay 16-byte aligned for bulk copies and double2 access
 
-// ---- shared epilogue pieces ---------------------------------------------------------------------------
 // bit mt*2+nt of the mask: the warp's 8x8 DMMA tile (mt, nt) has work (inside n x n, not strictly above the
 // diagonal of a diagonal tile)
 __device__ __forceinline__ unsigned tile_mask(int i0, int j0, int wr, int wc, int n, bool diag) {
@@ -35,103 +31,6 @@ __device__ __forceinline__ unsigned tile_mask(int i0, int j0, int wr, int wc, in
         }
     return m;
 }
-
-// P tile -> accumulator layout (lane g = lane>>2, q = lane&3 holds rows .. + g, columns .. + 2q, 2q+1)
-__device__ __forceinline__ void load_p_frags(const double* __restrict__ P, int ld, int n, int i0, int j0, int wr, int wc,
-                                             int g, int q, double (&pf)[4][2][2]) {
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt) {
-        const int gi = i0 + wr * 32 + mt * 8 + g;
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt) {
-            const int gj = j0 + wc * 16 + nt * 8 + 2 * q;
-            double2 val = make_double2(0.0, 0.0);
-            if (gi < n && gj < ld) val = *reinterpret_cast<const double2*>(P + (size_t)gi * ld + gj);
-            pf[mt][nt][0] = val.x; pf[mt][nt][1] = val.y;
-        }
-    }
-}
-
-// J on the P tile of tile column 0: the warps holding columns 0..7 (wc == 0, nt == 0) exchange them through
-// a [64][9] strip; 64 threads apply [c3 c4 c5 c6] <- [c3 c4 c5 c6] Jn' per row and, for tile (0,0), rows 3..6 <-
-// Jn * rows of the 8x8 corner.  `sync` is the barrier over the participating warps.
-template <typename Sync>
-__device__ __forceinline__ void apply_j_col0(double* strip, const double* __restrict__ Jn, bool diag, int wr, int wc, int g,
-                                             int q, int tid, double (&pf)[4][2][2], Sync sync) {
-    if (wc == 0) {
-#pragma unroll
-        for (int mt = 0; mt < 4; ++mt) {
-            strip[(wr * 32 + mt * 8 + g) * 9 + 2 * q] = pf[mt][0][0];
-            strip[(wr * 32 + mt * 8 + g) * 9 + 2 * q + 1] = pf[mt][0][1];
-        }
-    }
-    sync();
-    if (tid < TM) {
-        const int r = tid;
-        const double c3 = strip[r * 9 + 3], c4 = strip[r * 9 + 4], c5 = strip[r * 9 + 5], c6 = strip[r * 9 + 6];
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-            strip[r * 9 + 3 + a] = c3 * Jn[a * 4 + 0] + c4 * Jn[a * 4 + 1] + c5 * Jn[a * 4 + 2] + c6 * Jn[a * 4 + 3];
-    }
-    sync();
-    if (diag) {
-        if (tid < 8) {
-            const int c = tid;
-            const double r3 = strip[3 * 9 + c], r4 = strip[4 * 9 + c], r5 = strip[5 * 9 + c], r6 = strip[6 * 9 + c];
-#pragma unroll
-            for (int a = 0; a < 4; ++a)
-                strip[(3 + a) * 9 + c] = Jn[a * 4 + 0] * r3 + Jn[a * 4 + 1] * r4 + Jn[a * 4 + 2] * r5 + Jn[a * 4 + 3] * r6;
-        }
-        sync();
-    }
-    if (wc == 0) {
-#pragma unroll
-        for (int mt = 0; mt < 4; ++mt) {
-            pf[mt][0][0] = strip[(wr * 32 + mt * 8 + g) * 9 + 2 * q];
-            pf[mt][0][1] = strip[(wr * 32 + mt * 8 + g) * 9 + 2 * q + 1];
-        }
-    }
-    sync();  // the strip is free again
-}
-
-// C = P - acc, stored with its mirror image straight from the accumulator fragments (lanes with equal q cover
-// 64-byte runs).  Diagonal tiles: the lower triangle is authoritative, the upper one its mirror.
-__device__ __forceinline__ void store_tile(double* __restrict__ P, int ld, int n, int i0, int j0, int wr, int wc, int g, int q,
-                                           bool diag, unsigned onmask, const double (&pf)[4][2][2],
-                                           const double (&acc)[8][2]) {
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt) {
-        const int gi = i0 + wr * 32 + mt * 8 + g;
-        if (gi >= n) continue;
-#pragma unroll
-        for (int nt = 0; nt < 2; ++nt) {
-            if (!(onmask & (1u << (mt * 2 + nt)))) continue;
-            const int gj = j0 + wc * 16 + nt * 8 + 2 * q;
-            const double c0 = pf[mt][nt][0] - acc[mt * 2 + nt][0];
-            const double c1 = pf[mt][nt][1] - acc[mt * 2 + nt][1];
-            if (!diag) {
-                if (gj + 1 < n) {
-                    *reinterpret_cast<double2*>(P + (size_t)gi * ld + gj) = make_double2(c0, c1);
-                    P[(size_t)gj * ld + gi] = c0;
-                    P[(size_t)(gj + 1) * ld + gi] = c1;
-                } else if (gj < n) {
-                    P[(size_t)gi * ld + gj] = c0;
-                    P[(size_t)gj * ld + gi] = c0;
-                }
-            } else {
-                if (gj <= gi && gj < n) {
-                    P[(size_t)gi * ld + gj] = c0;
-                    if (gj < gi) P[(size_t)gj * ld + gi] = c0;
-                }
-                if (gj + 1 <= gi && gj + 1 < n) {
-                    P[(size_t)gi * ld + gj + 1] = c1;
-                    if (gj + 1 < gi) P[(size_t)(gj + 1) * ld + gi] = c1;
-                }
-            }
-        }
-    }
-}
-
 
 // ---- K chunk: acc += A' B over n4 steps of 4 rows of the staged panels ------------------------------------
 // `a` / `b` point at this lane's first fragment element of the stage (q*TPAD + warp offset + g).  A warp whose
@@ -213,7 +112,7 @@ struct TriW {
 #pragma unroll
         for (int i = 0; i < NA + NBK; ++i) {
             const int r = (i < NA) ? RA : RB, c = (i < NA) ? CA + i : CB + i - NA;
-            double2* xp = reinterpret_cast<double2*>(x + r * 8 * XP_ + c * 8);
+            double2* xp = reinterpret_cast<double2*>(x + r * 8 * XP + c * 8);
             double2 pv = *xp;
             pv.x -= acc[i][0];
             pv.y -= acc[i][1];
@@ -266,7 +165,7 @@ struct StripW {
     static __device__ __forceinline__ void update(double* __restrict__ x, const double (&acc)[8][2]) {
 #pragma unroll
         for (int rb = 0; rb < NRB; ++rb) {
-            double2* xp = reinterpret_cast<double2*>(x + rb * 8 * XP_);
+            double2* xp = reinterpret_cast<double2*>(x + rb * 8 * XP);
             double2 pv = *xp;
             pv.x -= acc[rb][0];
             pv.y -= acc[rb][1];
@@ -286,79 +185,7 @@ struct StripW {
         default: CALL(StripW<8>); break;          \
     }
 
-// ---- one CTA per tile, cp.async ring ------------------------------------------------------------------
-__global__ void __launch_bounds__(256, 3) k_downdate_tile(DevView v) {
-    extern __shared__ __align__(16) double dsm[];
-    const int b = blockIdx.y;
-    const int k = v.ktot[b];
-    if (k == 0) return;
-    const int n = v.nstate[b];
-    const int e = blockIdx.x;
-    int ti = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-    while ((ti + 1) * (ti + 2) / 2 <= e) ++ti;
-    while (ti * (ti + 1) / 2 > e) --ti;
-    const int tj = e - ti * (ti + 1) / 2;
-    const int i0 = ti * TM, j0 = tj * TM;
-    if (i0 >= n) return;
-    const int ld = v.ld, kmax = v.wrows;   // W panel stride (rows)
-    const double* __restrict__ W = v.W + (size_t)b * v.wstride;
-    double* __restrict__ P = v.P + (size_t)b * v.nmax * ld;
-    const bool diag = (ti == tj);
-    double* As = dsm;                            // [NSTAGE][TK][TPAD]
-    double* Bs = dsm + NSTAGE * TK * TPAD;       // [NSTAGE][TK][TPAD]
-    double* strip = Bs + NSTAGE * TK * TPAD;     // [64][9]
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int wr = warp >> 2, wc = warp & 3, g = lane >> 2, q = lane & 3;
-
-    double pf[4][2][2];
-    load_p_frags(P, ld, n, i0, j0, wr, wc, g, q, pf);
-    const int nk = (k + TK - 1) / TK;
-    const int lr = tid >> 5, lcc = (tid & 31) * 2;
-    const bool cola = (i0 + lcc < ld), colb = (j0 + lcc < ld);
-    const double* __restrict__ wa = W + w_at(kmax, lr, i0 + lcc);   // panel-major W: row stride EKF_WPAD inside a panel
-    const double* __restrict__ wb = W + w_at(kmax, lr, j0 + lcc);
-    const int soff = lr * TPAD + lcc;
-    auto load_stage = [&](int st, int t0) {
-        double* as = As + st * TK * TPAD + soff;
-        double* bs = Bs + st * TK * TPAD + soff;
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-            const int tt = t0 + lr + 8 * j;
-            const bool oka = (tt < k) && cola;
-            cp_async16(as + 8 * j * TPAD, oka ? wa + (size_t)(t0 + 8 * j) * EKF_WPAD : W, oka ? 16 : 0);
-            if (!diag) {
-                const bool okb = (tt < k) && colb;
-                cp_async16(bs + 8 * j * TPAD, okb ? wb + (size_t)(t0 + 8 * j) * EKF_WPAD : W, okb ? 16 : 0);
-            }
-        }
-    };
-    double acc[8][2];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) acc[i][0] = acc[i][1] = 0.0;
-    const unsigned onmask = tile_mask(i0, j0, wr, wc, n, diag);
-    const int aoff = q * TPAD + wr * 32 + g, boff = q * TPAD + wc * 16 + g;
-
-#pragma unroll
-    for (int st = 0; st < NSTAGE - 1; ++st) {
-        if (st < nk) load_stage(st, st * TK);
-        cp_async_commit();
-    }
-    for (int it = 0; it < nk; ++it) {
-        cp_async_wait<NSTAGE - 2>();
-        __syncthreads();
-        if (it + NSTAGE - 1 < nk) load_stage((it + NSTAGE - 1) % NSTAGE, (it + NSTAGE - 1) * TK);
-        cp_async_commit();
-        const double* as = As + (it % NSTAGE) * TK * TPAD;
-        const double* bs = diag ? as : Bs + (it % NSTAGE) * TK * TPAD;
-        mma_chunk(as + aoff, bs + boff, min(TK / 4, (k - it * TK + 3) >> 2), onmask, acc);  // the tail panel stops at k (rounded to 4)
-    }
-    cp_async_wait<0>();
-    if (tj == 0)
-        apply_j_col0(strip, v.jn + (size_t)b * 16, diag, wr, wc, g, q, tid, pf, [] { __syncthreads(); });
-    store_tile(P, ld, n, i0, j0, wr, wc, g, q, diag, onmask, pf, acc);
-}
-
-// ---- persistent, warp-specialised, with epilogue warps (default) ----------------------------------------
+// ---- persistent, warp-specialised, with epilogue warps ----------------------------------------------------
 // Roles per CTA (13 warps, 2 CTAs per SM); X = one shared [64][XP] tile buffer:
 //   warp  8     producer: streams the W panels with bulk copies through the mbarrier ring (one per panel and stage).
 //   warps 0-7   consumers: K loop; then J on tile column 0 of X (the prefetched P tile), X <- X - acc, and straight on
@@ -372,7 +199,6 @@ __global__ void __launch_bounds__(256, 3) k_downdate_tile(DevView v) {
 // and no P value is held in registers across the K loop.
 #define WS2_EPI 4
 #define WS2_THREADS ((WS_CONSUMERS + 1 + WS2_EPI) * 32)
-#define XP XP_  // row pitch of X in doubles (66): rows stay 16-byte aligned for bulk copies and double2 access
 
 __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 2, 128;" ::: "memory"); }
 __device__ __forceinline__ void cons_bar() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
@@ -402,7 +228,6 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
     unsigned long long* pfull = empty + S;   // [NX] P tile landed in X[j]
     unsigned long long* cfull = pfull + NX;  // [NX] X[j] holds P - acc
     int2* meta = reinterpret_cast<int2*>(cfull + NX);                                  // [M]  {ktot, n}
-    unsigned* lut = reinterpret_cast<unsigned*>(meta + M);                            // [T]  ti<<16|tj
     const int ld = v.ld, kmax = v.wrows;   // W panel stride (rows)
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long G = gridDim.x;
@@ -411,12 +236,6 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
         int2 kn = make_int2(0, 0);
         if (t < total) { const int b = b0 + (int)(t / T); kn = make_int2(v.ktot[b], v.nstate[b]); }
         meta[m] = kn;
-    }
-    for (int e = tid; e < T; e += blockDim.x) {
-        int ti = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-        while ((ti + 1) * (ti + 2) / 2 <= e) ++ti;
-        while (ti * (ti + 1) / 2 > e) --ti;
-        lut[e] = ((unsigned)ti << 16) | (unsigned)(e - ti * (ti + 1) / 2);
     }
     if (tid == 0) {
         for (int s2 = 0; s2 < S; ++s2) { mbar_init(full + s2, 32); mbar_init(empty + s2, WS_CONSUMERS); }
@@ -434,7 +253,7 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
         // has the padded [TK][TPAD] shared-memory layout -> one bulk copy per panel and stage, issued by lane 0.
         unsigned cnt = 0;
         for (int m = 0; m < Mreal; ++m) {
-            const DTile L = decode_tile(meta, lut, m, Mreal, blockIdx.x + (long long)m * G, T);
+            const DTile L = decode_tile(meta, m, Mreal, blockIdx.x + (long long)m * G, T);
             if (L.nk == 0) continue;
             const double* __restrict__ W = v.W + (size_t)(b0 + L.b) * v.wstride;
             const double* __restrict__ wa = W + w_at(kmax, 0, L.i0);
@@ -473,7 +292,7 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
         const int xoff = (wr * 32 + g) * XP + wc * 16 + 2 * q;
         unsigned cnt = 0, tiles = 0;
         for (int cm = 0; cm < Mreal; ++cm) {
-            const DTile C = decode_tile(meta, lut, cm, Mreal, blockIdx.x + (long long)cm * G, T);
+            const DTile C = decode_tile(meta, cm, Mreal, blockIdx.x + (long long)cm * G, T);
             if (C.nk == 0) continue;
             // warp layout of this tile: 0 = 2x4 grid of 32x16 (full tiles; masked path for the partial last diagonal tile),
             // 1 = STRIP (off-diagonal tile with fewer than 64 rows), 2 = TRI (full diagonal tile)
@@ -561,7 +380,7 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
     int pm = -1;
     DTile Pn;
     auto next_valid = [&](int m, DTile& t) {
-        do { ++m; t = decode_tile(meta, lut, m, Mreal, blockIdx.x + (long long)m * G, T); } while (m < Mreal && t.nk == 0);
+        do { ++m; t = decode_tile(meta, m, Mreal, blockIdx.x + (long long)m * G, T); } while (m < Mreal && t.nk == 0);
         return m;
     };
 #pragma unroll
@@ -617,6 +436,14 @@ __global__ void __launch_bounds__(WS2_THREADS, 2) k_downdate_ws2(DevView v, int 
     }
 }
 
+// shared memory of k_downdate_ws2<S, NX> besides its tile metadata: the W ring, the P tile buffers and the mbarriers
+constexpr size_t ws2_fixed_smem(int S, int NX) {
+    return sizeof(double) * (2 * S * TK * TPAD + NX * TM * XP) + sizeof(unsigned long long) * (2 * S + 2 * NX);
+}
+constexpr size_t WS2_SMEM_BUDGET = 111 * 1024;   // two CTAs per SM
+static_assert(ws2_fixed_smem(4, 1) + 64 * sizeof(int2) <= WS2_SMEM_BUDGET && ws2_fixed_smem(2, 2) + 64 * sizeof(int2) <= WS2_SMEM_BUDGET,
+              "k_downdate_ws2 leaves no room for tile metadata");
+
 void launch_downdate(ekfslam_ctx* c, int slot) {
     DevView& v = c->v;
     const int sms = c->sm_count;   // of the context's own device (a process may drive several GPUs)
@@ -626,37 +453,26 @@ void launch_downdate(ekfslam_ctx* c, int slot) {
     // ring depth / P buffers by update kind: the hi update and the camera-state update stack few rows (short K loops,
     // the kernel streams P), the li update many.
     const bool cfgB = slot != KT_DOWNDATE;
-    const int S = cfgB ? 2 : 4, NX = cfgB ? 2 : 1;
+    const size_t fixed = cfgB ? ws2_fixed_smem(2, 2) : ws2_fixed_smem(4, 1);
     // filters are processed in groups small enough for the per-CTA tile metadata (8 B per tile) to stay
     // within the shared-memory budget of two CTAs per SM
     const long long ctas_full = (long long)sms * 2;
-    const size_t fixed = sizeof(double) * (2 * S * TK * TPAD + NX * TM * XP) + sizeof(unsigned long long) * (2 * S + 2 * NX) +
-                         sizeof(unsigned) * T;
-    const size_t budget = 111 * 1024;
-    if (fixed + 64 * sizeof(int2) <= budget) {
-        const long long Mcap = (long long)((budget - fixed) / sizeof(int2));
-        long long bgroup = (Mcap * ctas_full) / T;
-        if (bgroup < 1) bgroup = 1;
-        const char* eg = getenv("EKFSLAM_DD_GROUP");   // =g: at most g filters per launch (exercises the grouping in tests)
-        const long long force_group = eg ? atoll(eg) : 0;
-        if (force_group > 0 && force_group < bgroup) bgroup = force_group;
-        for (long long b0 = 0; b0 < v.B; b0 += bgroup) {
-            const long long nb = (v.B - b0 < bgroup) ? (v.B - b0) : bgroup;
-            const long long total = (long long)T * nb;
-            const long long ctas = total < ctas_full ? total : ctas_full;
-            const int M = (int)((total + ctas - 1) / ctas);
-            const size_t sm2 = fixed + sizeof(int2) * M;
-            if (cfgB) ENSURE_DYN_SMEM((k_downdate_ws2<2, 2>), sm2, c->device);
-            else ENSURE_DYN_SMEM((k_downdate_ws2<4, 1>), sm2, c->device);
-            if (cfgB) k_downdate_ws2<2, 2><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
-            else k_downdate_ws2<4, 1><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
-            if (b0 > 0) c->launches++;
-        }
-        return;
+    const long long Mcap = (long long)((WS2_SMEM_BUDGET - fixed) / sizeof(int2));
+    long long bgroup = (Mcap * ctas_full) / T;
+    if (bgroup < 1) bgroup = 1;   // one filter beyond the budget (n_max > ~55 000 on 148 SMs) runs at one CTA per SM
+    const char* eg = getenv("EKFSLAM_DD_GROUP");   // =g: at most g filters per launch (exercises the grouping in tests)
+    const long long force_group = eg ? atoll(eg) : 0;
+    if (force_group > 0 && force_group < bgroup) bgroup = force_group;
+    for (long long b0 = 0; b0 < v.B; b0 += bgroup) {
+        const long long nb = (v.B - b0 < bgroup) ? (v.B - b0) : bgroup;
+        const long long total = (long long)T * nb;
+        const long long ctas = total < ctas_full ? total : ctas_full;
+        const int M = (int)((total + ctas - 1) / ctas);
+        const size_t sm2 = fixed + sizeof(int2) * M;
+        if (cfgB) ENSURE_DYN_SMEM((k_downdate_ws2<2, 2>), sm2, c->device);
+        else ENSURE_DYN_SMEM((k_downdate_ws2<4, 1>), sm2, c->device);
+        if (cfgB) k_downdate_ws2<2, 2><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
+        else k_downdate_ws2<4, 1><<<(unsigned)ctas, WS2_THREADS, sm2, c->stream>>>(v, T, (int)b0, total, M);
+        if (b0 > 0) c->launches++;
     }
-    // the tile table does not fit (li <4,1>: T > 2412, i.e. n_max > 4352; hi <2,2>: T > 2672, n_max > 4608): one CTA per tile
-    const size_t sm = sizeof(double) * (2 * NSTAGE * TK * TPAD + TM * 9);
-    ENSURE_DYN_SMEM(k_downdate_tile, sm, c->device);
-    dim3 gd(T, v.B);
-    k_downdate_tile<<<gd, 256, sm, c->stream>>>(v);
 }

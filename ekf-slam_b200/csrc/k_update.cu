@@ -10,19 +10,11 @@
 //
 // Kernels: k_upd_S (select + stack S, nu) -> k_chol (blocked Cholesky, inv(L), y) ->
 //          k_gemm (W = inv(L) G_sel, triangular GEMM on DMMA; also x+, q normalisation, normJac) ->
-//          k_wfix (W <- W J', bookkeeping) -> k_downdate* (P <- J P J' - W'W, k_downdate.cu).
+//          k_wfix (W <- W J', bookkeeping) -> k_downdate_ws2 (P <- J P J' - W'W, k_downdate.cu).
 #include "model.cuh"
 #include "tc_common.cuh"
 
 #define NB 16
-
-// index e of a lower triangle stored by rows -> (r, c), c <= r
-__device__ __forceinline__ void tri_unrank(int e, int& r, int& c) {
-    r = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
-    while ((r + 1) * (r + 2) / 2 <= e) ++r;
-    while (r * (r + 1) / 2 > e) --r;
-    c = e - r * (r + 1) / 2;
-}
 
 // S = G_sel H_sel' + I, lower triangle at feature-pair granularity: pair e -> (fa >= fb) -> one 2x2 block.
 // STAGED: the per-feature operands of the pair loop (feature index, state offset, block width, compact Jacobian) come from
@@ -513,10 +505,8 @@ __global__ void __launch_bounds__(CHS_T, MINB) k_chol_sm(DevView v) {
             const int mt = (m + 3) / 4;
             const int ntile = mt * (mt + 1) / 2;
             for (int e = tid; e < ntile; e += CHS_T) {
-                int ti = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                while ((ti + 1) * (ti + 2) / 2 <= e) ++ti;
-                while (ti * (ti + 1) / 2 > e) --ti;
-                const int tj = e - ti * (ti + 1) / 2;
+                int ti, tj;
+                tri_unrank(e, ti, tj);
                 double acc[4][4];
 #pragma unroll
                 for (int a = 0; a < 4; ++a)

@@ -1,5 +1,5 @@
 // Shared building blocks of the tensor-core kernels (k_w, k_downdate*): DMMA wrapper, cp.async ring
-// helpers, mbarrier / bulk-copy wrappers, lower-triangle tile decoding; and the 16-wide warp Cholesky of the
+// helpers, mbarrier / bulk-copy wrappers, lower-triangle unranking and tile decoding; and the 16-wide warp Cholesky of the
 // update's diagonal blocks.
 #pragma once
 #include "common.cuh"
@@ -83,22 +83,30 @@ __device__ __forceinline__ bool chol16_warp(double* __restrict__ Blk, int pitch,
 }
 
 
+// index e of a lower triangle stored by rows -> (r, c), c <= r.  The float square root is only a guess; the two loops
+// correct it, so the result is exact for any e.
+__device__ __forceinline__ void tri_unrank(int e, int& r, int& c) {
+    r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
+    while ((r + 1) * (r + 2) / 2 <= e) ++r;
+    while (r * (r + 1) / 2 > e) --r;
+    c = e - r * (r + 1) / 2;
+}
+
 struct DTile {
     int b, i0, j0, k, n, nk;
     bool diag, col0;
 };
 
-// tile m of this CTA (global tile t = blockIdx.x + m*G): metadata comes from shared memory
-// (meta[m] = {k, n} of the tile's filter, lut[e] = ti<<16|tj), never from a dependent global load
-__device__ __forceinline__ DTile decode_tile(const int2* meta, const unsigned* lut, int m, int M, long long t, int T,
-                                             int tile = TM) {
+// tile m of this CTA (global tile t = blockIdx.x + m*G, filter t / T, lower-triangle tile t % T): the filter's
+// metadata comes from shared memory (meta[m] = {k, n}), never from a dependent global load
+__device__ __forceinline__ DTile decode_tile(const int2* meta, int m, int M, long long t, int T) {
     DTile d;
     d.nk = 0; d.b = 0; d.i0 = 0; d.j0 = 0; d.k = 0; d.n = 0; d.diag = false; d.col0 = false;
     if (m >= M) return d;
     d.b = (int)(t / T);
-    const unsigned e = lut[(int)(t - (long long)d.b * T)];
-    const int ti = (int)(e >> 16), tj = (int)(e & 0xffffu);
-    d.i0 = ti * tile; d.j0 = tj * tile;
+    int ti, tj;
+    tri_unrank((int)(t - (long long)d.b * T), ti, tj);
+    d.i0 = ti * TM; d.j0 = tj * TM;
     d.diag = (ti == tj); d.col0 = (tj == 0);
     const int2 kn = meta[m];
     d.k = kn.x; d.n = kn.y;
