@@ -12,7 +12,7 @@
 //     k_cb_trail      S_ab -= L_aj L_bj' for the lower tiles behind the panel
 //   inverse, divide and conquer over block pairs [A 0; C D] -> [inv(A) 0; -inv(D) C inv(A), inv(D)], doubling the
 //   block size per level (2 launches per level, every output tile independent):
-//     k_cb_inv<0>     T = C inv(A)     (T parked in the unused UPPER triangle of the S buffer)
+//     k_cb_inv<0>     T = C inv(A)     (T' parked in the unused UPPER triangle of the S buffer)
 //     k_cb_inv<1>     X_C = -inv(D) T
 // followed by the existing y = X nu / inv(S) nu kernels (k_mk_y, k_mk_cv, k_mk_fin in k_update.cu).
 // Rows / columns >= k of a filter behave as an identity extension (loads are masked, stores are clipped), so filters
@@ -76,6 +76,23 @@ __device__ __forceinline__ void cb_zero(double (&acc)[4][2][2]) {
     for (int mi = 0; mi < 4; ++mi)
 #pragma unroll
         for (int ni = 0; ni < 2; ++ni) { acc[mi][ni][0] = 0.0; acc[mi][ni][1] = 0.0; }
+}
+
+// acc' -> dst block (c0, r0): element (i, j) of the block at row r0 of acc goes to dst[c0 + j][r0 + i], for r0 + i < k.
+// Parking T transposed keeps every column of T (rows r0 + i >= k of T only ever multiply zeros); parked as is, the block
+// column of T at c0 = 64 ti would be clipped at kmax when kmax < 64 (ti + 1), losing columns T needs.
+__device__ __forceinline__ void cb_store_t(double* __restrict__ dst, int kmax, int k, int r0, int c0, const double (&acc)[4][2][2]) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int wr = warp >> 2, wc = warp & 3, g = lane >> 2, q = lane & 3;
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < 2; ++ni) {
+            const int gi = r0 + wr * 32 + mi * 8 + g, gj = c0 + wc * 16 + ni * 8 + 2 * q;
+            if (gi >= k) continue;
+            dst[(size_t)gj * kmax + gi] = acc[mi][ni][0];
+            dst[(size_t)(gj + 1) * kmax + gi] = acc[mi][ni][1];
+        }
 }
 
 // dst block (r0, c0) = alpha * acc (+ beta_one * old), clipped to [0,k)^2
@@ -271,8 +288,8 @@ __global__ void __launch_bounds__(256) k_cb_trail(DevView v, int j0) {
 // ---------------------------------------------------------------------------------------
 // triangular inverse, one level of the divide and conquer.  Blocks are 64 wide; at level s the diagonal blocks of
 // 2s have known inverses for their two halves A = [2ps, 2ps+s), D = [2ps+s, 2ps+2s) and the coupling block C = L[D, A]
-// becomes X[D, A] = -inv(D) C inv(A).  phase 0: T[ti][tj] = sum_{t in A, t >= tj} L[ti][t] X[t][tj], stored at block
-// (tj, ti) of the S buffer (upper triangle, unused);  phase 1: X[ti][tj] = -sum_{t in D, t <= ti} X[ti][t] T[t][tj].
+// becomes X[D, A] = -inv(D) C inv(A).  phase 0: T[ti][tj] = sum_{t in A, t >= tj} L[ti][t] X[t][tj], stored transposed
+// at block (tj, ti) of the S buffer (upper triangle, unused);  phase 1: X[ti][tj] = -sum_{t in D, t <= ti} X[ti][t] T[t][tj].
 // grid = (nblk * s, B): blockIdx.x -> (ti, o), tj = pair base + o
 // ---------------------------------------------------------------------------------------
 template <int phase>
@@ -300,14 +317,14 @@ __global__ void __launch_bounds__(256) k_cb_inv(DevView v, int s) {
             __syncthreads();
             cb_mma<false>(acc, As, Bs);
         }
-        cb_store(S, kmax, kmax, tj * CB, ti * CB, acc, 1.0, false); // park T in the upper triangle, whole block
+        cb_store_t(S, kmax, k, ti * CB, tj * CB, acc);              // park T' at block (tj, ti), upper triangle
     } else {
         for (int t = base + s; t <= ti; ++t) {
             __syncthreads();
             cb_load(As, X, kmax, k, ti * CB, t * CB, t == ti);      // X[ti][t]
-            cb_load(Bs, S, kmax, kmax, tj * CB, t * CB, false);     // T[t][tj] parked at (tj, t)
+            cb_load(Bs, S, kmax, k, tj * CB, t * CB, false);        // T[t][tj]' parked at (tj, t)
             __syncthreads();
-            cb_mma<false>(acc, As, Bs);
+            cb_mma<true>(acc, As, Bs);
         }
         cb_store(X, kmax, k, ti * CB, tj * CB, acc, -1.0, false);
     }
