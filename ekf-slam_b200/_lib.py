@@ -55,6 +55,10 @@ EVAL_FIELDS = [f[0] for f in Eval._fields_]
 EVAL_CAM_NOT_SPD, EVAL_NO_TRUTH, EVAL_NOT_EVALUABLE = 1, 2, 4
 # per-filter status of ekfslam_update_camera
 CAM_APPLIED, CAM_OFF, CAM_GATED, CAM_NOT_SPD = 0, 1, 2, 3
+# ekfslam_update_landmarks: landmarks per filter, per-landmark status, per-filter status
+LM_MAX = 16
+LM_USED, LM_NOT_OBSERVED, LM_NOT_VISIBLE, LM_GATED, LM_NOT_SPD, LM_ABSENT = 0, 1, 2, 3, 4, 5
+LMU_APPLIED, LMU_NONE, LMU_NOT_SPD = 0, 1, 2
 
 
 class WorldParams(C.Structure):
@@ -127,6 +131,12 @@ _SIGS = {
     "ekfslam_map_cartesian": (_I, [_P, _I, _I, _P, _P]),
     "ekfslam_update_camera": (_I, [_P, _I, _I, _I, _P, _P, _P, _P, C.c_double, _I]),
     "ekfslam_download_camera_update": (_I, [_P, _I, _I, _P, _P]),
+    "ekfslam_upload_landmarks": (_I, [_P, _I, _I, _I, _P, _P, _P, _P]),
+    "ekfslam_upload_landmark_obs": (_I, [_P, _I, _I, _P, _P]),
+    "ekfslam_world_landmark_obs": (_I, [_P, _I]),
+    "ekfslam_download_landmark_obs": (_I, [_P, _I, _I, _P, _P]),
+    "ekfslam_update_landmarks": (_I, [_P, C.c_double, C.c_double, _I]),
+    "ekfslam_download_landmark_update": (_I, [_P, _I, _I, _P, _P, _P, _P, _P, _P]),
     "ekfslam_device_ptr": (_P, [_P, C.c_char_p]),
     "ekfslam_enable_timing": (_I, [_P, _I]),
     "ekfslam_kernel_count": (_I, []),

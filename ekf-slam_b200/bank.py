@@ -33,6 +33,7 @@ class FilterBank:
         L.check(self.lib.ekfslam_create(C.byref(h), int(device), int(B), int(N_max), n_max))
         self._h = h
         self.B, self.N, self.n_max, self.device = int(B), int(N_max), n_max, int(device)
+        self._lm_L = 0    # landmarks per filter of the last upload_landmarks
         ld = C.c_int()
         L.check(self.lib.ekfslam_dims(self._h, None, None, None, C.byref(ld)))
         self.ld = ld.value
@@ -385,6 +386,65 @@ class FilterBank:
         nis, st = np.empty(nb), np.empty(nb, dtype=np.int32)
         L.check(self.lib.ekfslam_download_camera_update(self._h, b0, nb, _ptr(nis), _ptr(st)))
         return {"nis": nis, "status": st}
+
+    # -- known-landmark update (extension) ------------------------------------------------------
+    def upload_landmarks(self, pts, cov=None, tag=None, nlm=None, b0=0):
+        """Landmarks of filters [b0, b0+nb) (see ekfslam_upload_landmarks): pts [nb,L,3] world positions, cov [nb,L,6]
+        packed (xx, yx, yy, zx, zy, zz) or [nb,L,3,3] (None: exactly known), tag [nb,L] world points for
+        world_landmark_obs (None: -1), nlm [nb] landmarks in use (None: L).  L <= min(LM_MAX, N_max) becomes the
+        bank's landmark count."""
+        pts = _c(pts, np.float64)
+        if pts.ndim != 3 or pts.shape[2] != 3:
+            raise ValueError("pts must be [nb, L, 3]")
+        nb, Lm = pts.shape[:2]
+        if cov is not None:
+            cov = np.asarray(cov, dtype=np.float64)
+            if cov.shape == (nb, Lm, 3, 3):
+                cov = cov[..., [0, 1, 1, 2, 2, 2], [0, 0, 1, 0, 1, 2]]
+            cov = _c(cov, np.float64, (nb, Lm, 6))
+        tag = None if tag is None else _c(tag, np.int32, (nb, Lm))
+        nlm = None if nlm is None else _c(nlm, np.int32, (nb,))
+        L.check(self.lib.ekfslam_upload_landmarks(self._h, int(b0), nb, Lm, _ptr(pts), _ptr(cov), _ptr(tag), _ptr(nlm)))
+        self._lm_L = Lm
+
+    def upload_landmark_obs(self, uv, has=None, b0=0):
+        """This frame's observations: uv [nb,L,2] distorted pixels, has [nb,L] (None: all observed)."""
+        uv = _c(uv, np.float64)
+        if uv.ndim != 3 or uv.shape[2] != 2:
+            raise ValueError("uv must be [nb, L, 2]")
+        nb = uv.shape[0]
+        if self._lm_L and uv.shape[1] != self._lm_L:
+            raise ValueError("uv must have L = %d landmarks" % self._lm_L)
+        has = None if has is None else _c(has, np.uint8, uv.shape[:2])
+        L.check(self.lib.ekfslam_upload_landmark_obs(self._h, int(b0), nb, _ptr(uv), _ptr(has)))
+
+    def world_landmark_obs(self, t):
+        """Synthetic observations of frame t of the uploaded world for the tagged landmarks (stream-ordered)."""
+        L.check(self.lib.ekfslam_world_landmark_obs(self._h, int(t)))
+
+    def download_landmark_obs(self, b0=0, nb=None):
+        """The staged observations: uv [nb,L,2], has [nb,L] u8."""
+        nb = self.B - b0 if nb is None else nb
+        uv, has = np.empty((nb, self._lm_L or 1, 2)), np.empty((nb, self._lm_L or 1), dtype=np.uint8)
+        L.check(self.lib.ekfslam_download_landmark_obs(self._h, b0, nb, _ptr(uv), _ptr(has)))
+        return uv, has
+
+    def update_landmarks(self, std_px, gate=0.0, which=0):
+        """Known-landmark update of every filter (see ekfslam_update_landmarks): which=0 updates (x_k_k, P), which=1
+        (x_k_km1, P); gate <= 0: no chi-square gate.  Stream-ordered; results from download_landmark_update()."""
+        L.check(self.lib.ekfslam_update_landmarks(self._h, float(std_px), float(gate), int(which)))
+
+    def download_landmark_update(self, b0=0, nb=None):
+        """{"nis", "k", "status"} [nb] per filter (LMU_*; NIS NaN unless applied) and {"lm_status" [nb,L] (LM_*),
+        "lm_h" [nb,L,2], "lm_nis" [nb,L]} per landmark of the last update_landmarks."""
+        nb = self.B - b0 if nb is None else nb
+        Lm = self._lm_L or 1    # before any upload the call fails with ERR_STATE
+        out = {"nis": np.empty(nb), "k": np.empty(nb, dtype=np.int32), "status": np.empty(nb, dtype=np.int32),
+               "lm_status": np.empty((nb, Lm), dtype=np.int32), "lm_h": np.empty((nb, Lm, 2)),
+               "lm_nis": np.empty((nb, Lm))}
+        L.check(self.lib.ekfslam_download_landmark_update(self._h, b0, nb, *(_ptr(out[k]) for k in (
+            "nis", "k", "status", "lm_status", "lm_h", "lm_nis"))))
+        return out
 
     # -- stages (names follow the reference functions they replace) --------------------------
     def begin_frame(self):

@@ -98,7 +98,8 @@ static void kt_collect(ekfslam_ctx* c) {
 static const char* KT_NAMES[KT_COUNT] = {"k_begin_frame", "k_predict", "k_features", "k_hp", "k_innov", "k_ransac",
                                          "k_upd_S", "k_chol", "k_w", "k_downdate_hi", "k_downdate", "k_symmetrize",
                                          "k_add_features", "k_wfix", "k_w_hi", "k_chol_hi", "k_upd_S_hi",
-                                         "k_hp_rescue", "k_world", "k_eval", "k_cam_update", "k_downdate_cam"};
+                                         "k_hp_rescue", "k_world", "k_eval", "k_cam_update", "k_downdate_cam",
+                                         "k_lm_update", "k_downdate_lm"};
 
 template <typename T>
 static cudaError_t dalloc(T** p, size_t count, int64_t* total) {
@@ -281,7 +282,9 @@ int ekfslam_destroy(ekfslam_ctx* c) {
                     v.flags, v.mflags, v.foff, v.nstate, v.nfeat, v.counters, v.tag, v.sel, v.ksel, v.stats, v.nhyp_tab,
                     c->mm_del, c->mm_quota, c->det_n, c->det_uv, c->det_tag, c->world_points, c->world_poses,
                     c->ev.rec, c->ev.tot, c->ev.ferr, c->ev.fnees, c->ev.mp, c->ev.mc,
-                    c->cu.H, c->cu.z, c->cu.R, c->cu.on, c->cu.nis, c->cu.status};
+                    c->cu.H, c->cu.z, c->cu.R, c->cu.on, c->cu.nis, c->cu.status,
+                    c->lm.p, c->lm.C, c->lm.tag, c->lm.nlm, c->lm.uv, c->lm.has, c->lm.nis, c->lm.k, c->lm.status,
+                    c->lm.lm_status, c->lm.lm_h, c->lm.lm_nis};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (c->timer) {
@@ -1220,6 +1223,135 @@ int ekfslam_download_camera_update(ekfslam_ctx* c, int b0, int nb, double* nis, 
     if (!u.H) return fail(EKFSLAM_ERR_STATE, "no camera update yet (ekfslam_update_camera)");
     if (nis) CK(cudaMemcpyAsync(nis, u.nis + b0, sizeof(double) * nb, cudaMemcpyDeviceToHost, c->stream));
     if (status) CK(cudaMemcpyAsync(status, u.status + b0, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return EKFSLAM_OK;
+}
+
+// ---- known-landmark update (k_lm_update.cu) ---------------------------------------------------
+// Device arrays hold EKFSLAM_LM_MAX slots per filter; host arrays hold L (the context's count).  Copies between the
+// two pitches are 2-D copies: nb rows of L * w elements of `es` bytes.
+static cudaError_t lm_up(void* dev, const void* host, size_t es, int b0, int nb, int L, int w, cudaStream_t s) {
+    const size_t dp = es * EKFSLAM_LM_MAX * w, hp = es * L * w;
+    return cudaMemcpy2DAsync((char*)dev + dp * b0, dp, host, hp, hp, nb, cudaMemcpyHostToDevice, s);
+}
+static cudaError_t lm_down(void* host, const void* dev, size_t es, int b0, int nb, int L, int w, cudaStream_t s) {
+    const size_t dp = es * EKFSLAM_LM_MAX * w, hp = es * L * w;
+    return cudaMemcpy2DAsync(host, hp, (const char*)dev + dp * b0, dp, hp, nb, cudaMemcpyDeviceToHost, s);
+}
+
+int ekfslam_upload_landmarks(ekfslam_ctx* c, int b0, int nb, int L, const double* pts, const double* cov,
+                             const int32_t* tag, const int32_t* nlm) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    const int lmax = c->v.N < EKFSLAM_LM_MAX ? c->v.N : EKFSLAM_LM_MAX;   // W has 2 N_max rows per panel
+    if (L < 1 || L > lmax) return fail(EKFSLAM_ERR_INVALID, "L must be in [1, min(16, N_max)]");
+    if (!pts) return fail(EKFSLAM_ERR_INVALID, "pts is null");
+    if (nlm)
+        for (int i = 0; i < nb; ++i)
+            if (nlm[i] < 0 || nlm[i] > L) return fail(EKFSLAM_ERR_INVALID, "nlm must be in [0, L]");
+    DevLm& u = c->lm;
+    const size_t B = (size_t)c->v.B, S = B * EKFSLAM_LM_MAX;
+    if (!u.p) {   // first call: the buffers are allocated here, so a context that never uses landmarks holds none
+        cudaError_t er = cudaMalloc((void**)&u.p, sizeof(double) * 3 * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.C, sizeof(double) * 6 * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.tag, sizeof(int32_t) * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.nlm, sizeof(int32_t) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.uv, sizeof(double) * 2 * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.has, S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.nis, sizeof(double) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.k, sizeof(int32_t) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.status, sizeof(int32_t) * B);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.lm_status, sizeof(int32_t) * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.lm_h, sizeof(double) * 2 * S);
+        if (er == cudaSuccess) er = cudaMalloc((void**)&u.lm_nis, sizeof(double) * S);
+        if (er == cudaSuccess) er = cudaMemsetAsync(u.nlm, 0, sizeof(int32_t) * B, c->stream);   // filters never uploaded: none
+        if (er == cudaSuccess) er = cudaMemsetAsync(u.tag, 0xff, sizeof(int32_t) * S, c->stream);
+        if (er == cudaSuccess) er = cudaMemsetAsync(u.has, 0, S, c->stream);
+        if (er != cudaSuccess) {   // all or nothing: u.p != null means every buffer exists
+            for (void* q : {(void*)u.p, (void*)u.C, (void*)u.tag, (void*)u.nlm, (void*)u.uv, (void*)u.has, (void*)u.nis,
+                            (void*)u.k, (void*)u.status, (void*)u.lm_status, (void*)u.lm_h, (void*)u.lm_nis})
+                if (q) cudaFree(q);
+            u = DevLm();
+            cudaGetLastError();
+            return fail(er == cudaErrorMemoryAllocation ? EKFSLAM_ERR_NOMEM : EKFSLAM_ERR_CUDA,
+                        std::string("landmark buffers: ") + cudaGetErrorString(er));
+        }
+        c->bytes += (int64_t)((sizeof(double) * 14 + sizeof(int32_t) * 2 + 1) * S + (sizeof(double) + sizeof(int32_t) * 3) * B);
+    }
+    u.L = L;
+    const size_t n = (size_t)nb;
+    CK(lm_up(u.p, pts, sizeof(double), b0, nb, L, 3, c->stream));
+    if (cov) CK(lm_up(u.C, cov, sizeof(double), b0, nb, L, 6, c->stream));
+    else CK(cudaMemsetAsync(u.C + (size_t)b0 * EKFSLAM_LM_MAX * 6, 0, sizeof(double) * n * EKFSLAM_LM_MAX * 6, c->stream));
+    if (tag) CK(lm_up(u.tag, tag, sizeof(int32_t), b0, nb, L, 1, c->stream));
+    else CK(cudaMemsetAsync(u.tag + (size_t)b0 * EKFSLAM_LM_MAX, 0xff, sizeof(int32_t) * n * EKFSLAM_LM_MAX, c->stream));
+    if (nlm) CK(cudaMemcpyAsync(u.nlm + b0, nlm, sizeof(int32_t) * n, cudaMemcpyHostToDevice, c->stream));
+    else {   // a pageable source: the copy has taken the data when cudaMemcpyAsync returns
+        std::vector<int32_t> full(n, L);
+        CK(cudaMemcpyAsync(u.nlm + b0, full.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, c->stream));
+    }
+    return EKFSLAM_OK;
+}
+
+int ekfslam_upload_landmark_obs(ekfslam_ctx* c, int b0, int nb, const double* uv, const uint8_t* has) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    DevLm& u = c->lm;
+    if (!u.p) return fail(EKFSLAM_ERR_STATE, "no landmarks yet (ekfslam_upload_landmarks)");
+    if (!uv) return fail(EKFSLAM_ERR_INVALID, "uv is null");
+    CK(lm_up(u.uv, uv, sizeof(double), b0, nb, u.L, 2, c->stream));
+    if (has) CK(lm_up(u.has, has, 1, b0, nb, u.L, 1, c->stream));
+    else CK(cudaMemsetAsync(u.has + (size_t)b0 * EKFSLAM_LM_MAX, 1, (size_t)nb * EKFSLAM_LM_MAX, c->stream));
+    u.have_obs = 1;
+    return EKFSLAM_OK;
+}
+
+int ekfslam_world_landmark_obs(ekfslam_ctx* c, int t) {
+    NEED_CTX(c);
+    if (!c->world_points) return fail(EKFSLAM_ERR_STATE, "no world uploaded (ekfslam_world_upload)");
+    if (!c->lm.p) return fail(EKFSLAM_ERR_STATE, "no landmarks yet (ekfslam_upload_landmarks)");
+    if (t < 0 || t > c->world.T) return fail(EKFSLAM_ERR_INVALID, "frame index out of [0, T]");
+    launch_world_landmark_obs(c, t);
+    LAUNCHED();
+    c->lm.have_obs = 1;
+    return EKFSLAM_OK;
+}
+
+int ekfslam_download_landmark_obs(ekfslam_ctx* c, int b0, int nb, double* uv, uint8_t* has) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    const DevLm& u = c->lm;
+    if (!u.have_obs) return fail(EKFSLAM_ERR_STATE, "no landmark observations yet");
+    if (uv) CK(lm_down(uv, u.uv, sizeof(double), b0, nb, u.L, 2, c->stream));
+    if (has) CK(lm_down(has, u.has, 1, b0, nb, u.L, 1, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return EKFSLAM_OK;
+}
+
+int ekfslam_update_landmarks(ekfslam_ctx* c, double std_px, double gate, int which) {
+    NEED_CTX(c);
+    if (which != 0 && which != 1) return fail(EKFSLAM_ERR_INVALID, "which must be 0 (x_k_k) or 1 (x_k_km1)");
+    if (!(std_px >= 0.0) || !std::isfinite(std_px)) return fail(EKFSLAM_ERR_INVALID, "std_px must be finite and >= 0");
+    if (!c->lm.p || !c->lm.have_obs)
+        return fail(EKFSLAM_ERR_STATE, "no landmarks or observations yet (ekfslam_upload_landmarks / _obs)");
+    launch_lm_update(c, std_px, gate, which);
+    LAUNCHED();
+    c->lm.updated = 1;
+    return EKFSLAM_OK;
+}
+
+int ekfslam_download_landmark_update(ekfslam_ctx* c, int b0, int nb, double* nis, int32_t* k, int32_t* status,
+                                     int32_t* lm_status, double* lm_h, double* lm_nis) {
+    NEED_CTX(c);
+    if (check_range(c, b0, nb)) return EKFSLAM_ERR_INVALID;
+    const DevLm& u = c->lm;
+    if (!u.updated) return fail(EKFSLAM_ERR_STATE, "no landmark update yet (ekfslam_update_landmarks)");
+    if (nis) CK(cudaMemcpyAsync(nis, u.nis + b0, sizeof(double) * nb, cudaMemcpyDeviceToHost, c->stream));
+    if (k) CK(cudaMemcpyAsync(k, u.k + b0, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost, c->stream));
+    if (status) CK(cudaMemcpyAsync(status, u.status + b0, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost, c->stream));
+    if (lm_status) CK(lm_down(lm_status, u.lm_status, sizeof(int32_t), b0, nb, u.L, 1, c->stream));
+    if (lm_h) CK(lm_down(lm_h, u.lm_h, sizeof(double), b0, nb, u.L, 2, c->stream));
+    if (lm_nis) CK(lm_down(lm_nis, u.lm_nis, sizeof(double), b0, nb, u.L, 1, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     return EKFSLAM_OK;
 }

@@ -71,7 +71,7 @@ struct DevWorld {
 enum {
     KT_BEGIN_FRAME = 0, KT_PREDICT, KT_FEATURES, KT_HP, KT_INNOV, KT_RANSAC, KT_UPD_S, KT_CHOL, KT_W, KT_DOWNDATE_HI,
     KT_DOWNDATE, KT_SYMMETRIZE, KT_ADD_FEATURES, KT_WFIX, KT_W_HI, KT_CHOL_HI, KT_UPD_S_HI, KT_HP_RESCUE, KT_WORLD, KT_EVAL,
-    KT_CAM_UPDATE, KT_DOWNDATE_CAM, KT_COUNT
+    KT_CAM_UPDATE, KT_DOWNDATE_CAM, KT_LM_UPDATE, KT_DOWNDATE_LM, KT_COUNT
 };
 struct KTimer;
 
@@ -97,6 +97,25 @@ struct DevCamUpd {
     int32_t* status;      // [B]        EKFSLAM_CAM_*
     int m, b0, nb;        // rows and filter range of the last call
     double gate;          // <= 0: no gate
+};
+
+// known-landmark update (k_lm_update.cu); allocated on the first ekfslam_upload_landmarks, so a context that never
+// uses landmarks holds none of it.  Per-landmark arrays have EKFSLAM_LM_MAX slots per filter whatever L is.
+struct DevLm {
+    double* p;            // [B][16][3]  world position
+    double* C;            // [B][16][6]  position covariance, packed (xx, yx, yy, zx, zy, zz)
+    int32_t* tag;         // [B][16]     world point (synthetic observations), -1: none
+    int32_t* nlm;         // [B]
+    double* uv;           // [B][16][2]  observed pixel
+    uint8_t* has;         // [B][16]
+    double* nis;          // [B]
+    int32_t* k;           // [B]
+    int32_t* status;      // [B]         EKFSLAM_LMU_*
+    int32_t* lm_status;   // [B][16]     EKFSLAM_LM_*
+    double* lm_h;         // [B][16][2]
+    double* lm_nis;       // [B][16]
+    int L;                // landmarks per filter of the last upload
+    int have_obs, updated;
 };
 
 struct ekfslam_ctx {
@@ -137,6 +156,7 @@ struct ekfslam_ctx {
     double* own_zc; uint8_t* own_mflags; double* own_u; int own_n_u;
     DevEval ev;
     DevCamUpd cu;
+    DevLm lm;
 };
 
 // W is stored panel-major: element (row t, column c) of a filter lives at ((c / 64) * wrows + t) * EKF_WPAD + c % 64.
@@ -218,3 +238,7 @@ void launch_mm_plan(ekfslam_ctx* c, int min_features);
 void launch_eval(ekfslam_ctx* c, int mode, int t, int b0, int nb);
 // camera-state update of (x_k_k, P) (which 0) or (x_k_km1, P) (which 1) from the staged c->cu, then the downdate
 void launch_cam_update(ekfslam_ctx* c, int which);
+// known-landmark update of (x_k_k, P) (which 0) or (x_k_km1, P) (which 1) from c->lm, then the downdate
+void launch_lm_update(ekfslam_ctx* c, double std_px, double gate, int which);
+// synthetic landmark observations of frame t from the world (k_map.cu)
+void launch_world_landmark_obs(ekfslam_ctx* c, int t);

@@ -40,9 +40,10 @@ __device__ __forceinline__ double world_project(const DevCam& cam, const double*
     return hz;
 }
 
-__device__ __forceinline__ void world_gauss(const DevWorld& w, int b, int t, int id, double& n0, double& n1) {
-    const double u1 = world_u01(w.seed, b + w.b_offset, t, id, 1);
-    const double u2 = world_u01(w.seed, b + w.b_offset, t, id, 2);
+// Box-Muller pair from noise channels c1 and c1 + 1
+__device__ __forceinline__ void world_gauss(const DevWorld& w, int b, int t, int id, double& n0, double& n1, int c1 = 1) {
+    const double u1 = world_u01(w.seed, b + w.b_offset, t, id, c1);
+    const double u2 = world_u01(w.seed, b + w.b_offset, t, id, c1 + 1);
     const double rad = sqrt(-2.0 * log(1.0 - u1));
     double s, c;
     sincos(2.0 * 3.14159265358979323846 * u2, &s, &c);
@@ -179,6 +180,47 @@ __global__ void k_synth_uniforms(DevView v, DevWorld w, int t) {
     if (e >= v.B * v.n_u) return;
     const int b = e / v.n_u, i = e - b * v.n_u;
     v.u[e] = world_u01(w.seed, b + w.b_offset, t, i, 7);
+}
+
+// ---------------------------------------------------------------------------------------
+// landmark observations of frame t (ekfslam_world_landmark_obs): one thread per (filter, landmark slot).  Landmark j
+// with j < nlm[b] and a tag in [0, M) is that world point, seen as the candidates see it (visibility, outlier model,
+// pixel noise) but on noise channels 8..12, so its noise is independent of the candidate of the same point.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(128) k_synth_landmark_obs(int B, DevCam cam, DevWorld w, DevLm lm, int t) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= B * EKFSLAM_LM_MAX) return;
+    const int b = e / EKFSLAM_LM_MAX, j = e - b * EKFSLAM_LM_MAX;
+    double zx = 0.0, zy = 0.0;
+    uint8_t has = 0;
+    const int id = lm.tag[e];
+    if (j < lm.nlm[b] && id >= 0 && id < w.M) {
+        double ud, vd;
+        const double dep = world_project(cam, w.points + ((size_t)b * w.M + id) * 3, w.poses + ((size_t)t * B + b) * 7, ud, vd);
+        if (dep > 0.0 && ud > 0.0 && ud < cam.nCols && vd > 0.0 && vd < cam.nRows) {
+            const double u0 = world_u01(w.seed, b + w.b_offset, t, id, 8);
+            const double p_out = (id % w.flaky_mod == w.flaky_mod - 1) ? w.p_flaky : w.p_outlier;
+            if (u0 < p_out) {
+                zx = ud + (2.0 * world_u01(w.seed, b + w.b_offset, t, id, 11) - 1.0) * w.gross_px;
+                zy = vd + (2.0 * world_u01(w.seed, b + w.b_offset, t, id, 12) - 1.0) * w.gross_px;
+            } else {
+                double n0, n1;
+                world_gauss(w, b, t, id, n0, n1, 9);
+                zx = ud + n0 * w.noise_px;
+                zy = vd + n1 * w.noise_px;
+            }
+            has = 1;
+        }
+    }
+    lm.uv[2 * (size_t)e] = zx;
+    lm.uv[2 * (size_t)e + 1] = zy;
+    lm.has[e] = has;
+}
+
+void launch_world_landmark_obs(ekfslam_ctx* c, int t) {
+    const int tot = c->v.B * EKFSLAM_LM_MAX;
+    KScope ks(c, KT_WORLD);
+    k_synth_landmark_obs<<<(tot + 127) / 128, 128, 0, c->stream>>>(c->v.B, c->cam, c->world, c->lm, t);
 }
 
 void launch_world_uniforms(ekfslam_ctx* c, int t) {

@@ -414,8 +414,9 @@ class SynthWorld:
             vis = (dep > 0) & (zt[..., 0] > 0) & (zt[..., 0] < cam.nCols) & (zt[..., 1] > 0) & (zt[..., 1] < cam.nRows)
         return zt, vis
 
-    def _noise(self, b, t, w):
-        u = [world_uniform(self.seed, b + self.b_offset, t, w, c) for c in range(6)]
+    def _noise(self, b, t, w, c0=0):
+        """Uniforms of channels c0..c0+5 and the Box-Muller pair of channels c0+1, c0+2."""
+        u = [world_uniform(self.seed, b + self.b_offset, t, w, c0 + c) for c in range(6)]
         rad = np.sqrt(-2.0 * np.log(1.0 - u[1]))
         n0, n1 = rad * np.cos(2.0 * np.pi * u[2]), rad * np.sin(2.0 * np.pi * u[2])
         return u, n0, n1
@@ -442,6 +443,32 @@ class SynthWorld:
             has[b, :k] = vis[b, w]
             zc[b, :k][~vis[b, w]] = 0.0
         return zc, has
+
+    def landmark_obs(self, t, tags, nlm):
+        """Observations of known landmarks at frame t (numpy mirror of k_synth_landmark_obs): landmark j of filter b,
+        j < nlm[b], is world point tags[b, j] when that is in [0, M); it is observed when visible at the true pose of
+        frame t, with the candidates' outlier model and pixel noise drawn on noise channels 8..12 (independent of the
+        candidate of the same point).  tags [B,L], nlm [B].  Returns uv [B,L,2] (0 where not observed), has [B,L] u8."""
+        B, Lm = tags.shape
+        zt, vis = self.truth_pixels(t)
+        uv = np.zeros((B, Lm, 2))
+        has = np.zeros((B, Lm), dtype=np.uint8)
+        for b in range(B):
+            j = np.arange(Lm)
+            w = tags[b].astype(np.int64)
+            ok = (j < int(nlm[b])) & (w >= 0) & (w < self.M)
+            ok[ok] = vis[b, w[ok]]
+            if not ok.any():
+                continue
+            w = w[ok]
+            u, n0, n1 = self._noise(b, t, w, c0=8)
+            p_out = np.where(w % self.flaky_mod == self.flaky_mod - 1, self.p_flaky, self.p_outlier)
+            out = u[0] < p_out
+            zg = zt[b, w] + np.stack([(2 * u[3] - 1), (2 * u[4] - 1)], -1) * self.gross_px
+            zn = zt[b, w] + np.stack([n0, n1], -1) * self.noise_px
+            uv[b, ok] = np.where(out[:, None], zg, zn)
+            has[b, ok] = 1
+        return uv, has
 
     def uniforms(self, t, n_u):
         """RANSAC uniform stream of frame t, [B, n_u] — bit-identical to k_synth_uniforms (integer hash, exact scaling)."""

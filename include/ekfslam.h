@@ -374,6 +374,59 @@ int ekfslam_update_camera(ekfslam_ctx* ctx, int b0, int nb, int m, const double*
 /* last call's per-filter NIS [nb] and status [nb] (either may be NULL); ERR_STATE before the first call */
 int ekfslam_download_camera_update(ekfslam_ctx* ctx, int b0, int nb, double* nis, int32_t* status);
 
+/* ---- known-landmark update (EXTENSION: the reference has no such update) ---- */
+/* Pixel observations of points with known world coordinates (fiducial markers, surveyed ground-control points, points
+ * of a prior map) fix each filter's pose and scale.  The landmarks stay outside the state.
+ * Filter b has nlm[b] <= L landmarks, 1 <= L <= min(EKFSLAM_LM_MAX, N_max) (the update stacks k = 2 (landmarks used)
+ * rows in W, which has 2 N_max rows).  Landmark j has a world position p_j (3), an optional position covariance C_j
+ * packed (xx, yx, yy, zx, zy, zz) as in ekfslam_map_cartesian (NULL: exactly known) and an optional tag_j, the world
+ * point it is (ekfslam_world_landmark_obs only; -1: none).  Per frame it has a distorted pixel uv_j and a flag has_j.
+ * For every landmark with j < nlm[b] and has_j != 0, at the estimate x^:
+ *   h_j   = the prediction of mc/hi_cartesian.m:7-49 with y = p_j, including its +-60 deg field-of-view gate and its
+ *           in-image gate (not visible: the landmark is not used);
+ *   A_j   = columns 0..6 (r, q) and J_p = columns 7..9 (p) of the Cartesian Jacobian of mc/calculate_Hi_cartesian.m,
+ *           linearised at the predicted pixel h_j as in the reference;
+ *   R_j   = std_px^2 I2 + J_p C_j J_p',  S_j = A_j P[0:7,0:7] A_j' + R_j,  nu_j = uv_j - h_j;
+ *   gate  > 0: the landmark is used only if nu_j' inv(S_j) nu_j < gate (2 dof; the reference's value is 5.9915,
+ *           mc/rescue_hi_inliers.m:3); a 2x2 S_j that is not SPD means the landmark is not used.
+ * The used landmarks are stacked in landmark order: k = 2 (used) <= 32 rows, H = [A | 0], R block-diagonal, and the
+ * update is mc/update.m:3-32, computed the way the feature updates compute it:
+ *   S = H P H' + R = L L',  W = inv(L) (H P),  y = inv(L) nu,  x+ = x + W' y,  q+ <- q+/|q+|,
+ *   P+ = J P J' - (W J')' (W J') with J = blkdiag(I3, normJac(q+), I);  NIS = |y|^2 (k degrees of freedom).
+ * which: 0 updates (x_k_k, P), 1 updates (x_k_km1, P); the call orders are those of ekfslam_update_camera.
+ * Per landmark a status (EKFSLAM_LM_*), its h_j and its individual NIS are recorded: h_j is NaN where it was not
+ * formed (absent, not observed, not visible), the NIS where S_j was not formed or is not SPD.  Per filter a status
+ * (EKFSLAM_LMU_*): 0 applied, 1 nothing used (k = 0), 2 joint S not SPD or NIS not finite.  Statuses 1 and 2 leave
+ * every byte of that filter's state unchanged.  The cost is one pass of the covariance downdate over P.  Every call
+ * is stream-ordered, with no synchronisation (the downloads synchronise); the buffers are allocated on the first
+ * ekfslam_upload_landmarks. */
+#define EKFSLAM_LM_MAX 16
+enum { EKFSLAM_LM_USED = 0, EKFSLAM_LM_NOT_OBSERVED = 1, EKFSLAM_LM_NOT_VISIBLE = 2, EKFSLAM_LM_GATED = 3,
+       EKFSLAM_LM_NOT_SPD = 4, EKFSLAM_LM_ABSENT = 5 };
+enum { EKFSLAM_LMU_APPLIED = 0, EKFSLAM_LMU_NONE = 1, EKFSLAM_LMU_NOT_SPD = 2 };
+/* pts [nb][L][3], cov [nb][L][6] (NULL: exactly known), tag [nb][L] (NULL: -1), nlm [nb] in [0, L] (NULL: L).
+ * L is the context's landmark count from here on: observations and the per-landmark results are [nb][L].
+ * ERR_INVALID: L outside [1, min(16, N_max)], a bad [b0, b0+nb), a NULL pts, an nlm outside [0, L]. */
+int ekfslam_upload_landmarks(ekfslam_ctx* ctx, int b0, int nb, int L, const double* pts, const double* cov,
+                             const int32_t* tag, const int32_t* nlm);
+/* uv [nb][L][2] distorted pixels, has [nb][L] (NULL: all observed).  ERR_STATE before ekfslam_upload_landmarks. */
+int ekfslam_upload_landmark_obs(ekfslam_ctx* ctx, int b0, int nb, const double* uv, const uint8_t* has);
+/* synthetic observations of frame t from the world (ekfslam_world_upload), for every filter: landmark j with
+ * j < nlm[b] and tag_j in [0, M) is the world point tag_j, projected at the true pose of frame t (observed when its
+ * depth is > 0 and the pixel is inside the image), with the world's outlier model and pixel noise drawn on noise
+ * channels of its own (independent of the candidates of the same point).  ERR_STATE without a world or landmarks,
+ * ERR_INVALID for t outside [0, T]. */
+int ekfslam_world_landmark_obs(ekfslam_ctx* ctx, int t);
+/* the staged observations, uv [nb][L][2] and has [nb][L] (either may be NULL); ERR_STATE before any */
+int ekfslam_download_landmark_obs(ekfslam_ctx* ctx, int b0, int nb, double* uv, uint8_t* has);
+/* the update of every filter; std_px >= 0 (finite), gate <= 0: no gate.  ERR_INVALID: which not 0 or 1, std_px
+ * negative or not finite; ERR_STATE before landmarks and observations exist. */
+int ekfslam_update_landmarks(ekfslam_ctx* ctx, double std_px, double gate, int which);
+/* the last update's per-filter NIS [nb], k [nb], status [nb] and per-landmark status [nb][L], h [nb][L][2] and
+ * individual NIS [nb][L]; any pointer may be NULL.  ERR_STATE before the first ekfslam_update_landmarks. */
+int ekfslam_download_landmark_update(ekfslam_ctx* ctx, int b0, int nb, double* nis, int32_t* k, int32_t* status,
+                                     int32_t* lm_status, double* lm_h, double* lm_nis);
+
 /* ---- measurement hooks ------------------------------------------------------ */
 /* bracket every kernel launch with a CUDA event pair on the context's stream and accumulate the
  * elapsed time per kernel; enabling again resets the accumulators, on=0 removes the events */
